@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Guidance-step benchmark (contract in the task statement; numbers explained in DESIGN.md section "Measurement").
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload c2|target|c3|c1]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload c2|target|c3|c1] [--dump-outputs DIR]
 
 A "step" is ONE full CLIP-guided DDIM sampling step on synthetic inputs: the sampler's no-grad UNet forward, the
 guidance function (UNet forward with grad -> fused cutouts -> CLIP ViT fwd -> spherical loss+grad -> ViT dgrad ->
@@ -59,8 +59,22 @@ def parse_args():
     p.add_argument("--two-forwards", action="store_true", help="evaluate the UNet separately for the sampler and for cond_fn like the reference does")
     p.add_argument("--unet-layout", default="nhwc", choices=["nhwc", "nchw"],
                    help="nhwc (default): channels_last trunk + fused GroupNorm/scale-shift/SiLU kernels (csrc/unet_norm.cu); nchw: stock torch ops")
-    p.add_argument("--cpu-budget-s", type=float, default=150.0)
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR",
+                   help="after the timed steps, write what the last timed step returned (sample, pred_xstart) to DIR/<name>.npy as float32; "
+                        "the inputs are seeded, so two builds run with the same arguments can be compared output for output")
+    args = p.parse_args()
+    if args.steps < 1:
+        p.error("--steps must be at least 1")
+    return args
+
+
+def dump_outputs(directory, arrays):
+    """DIR/<name>.npy, float32, for every tensor of ``arrays`` (each one is [1, 3, size, size]: at most 7 MB per array)."""
+    import numpy as np
+
+    os.makedirs(directory, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), t.detach().float().cpu().numpy())
 
 
 class Cfg:
@@ -104,6 +118,11 @@ class ClockSampler:
     def stop(self):
         if self.proc is not None:
             self.proc.terminate()
+            try:  # reap it: the benchmark must not leave nvidia-smi behind
+                self.proc.wait(timeout=5)
+            except subprocess.TimeoutExpired:
+                self.proc.kill()
+                self.proc.wait()
             self.proc = None
 
     def summary(self, t0, t1, t_end=None):
@@ -202,7 +221,7 @@ def build_cpu_reference(wl, seed=0, world=1, scaling="weak"):
     def step(x, i):
         state["ct"] = i
         t = torch.full((1,), i, dtype=torch.long)
-        return diffusion.ddim_sample(unet, x, t, clip_denoised=False, denoised_fn=denoised_fn, cond_fn=cond_fn, model_kwargs={}, eta=0.8)["sample"]
+        return diffusion.ddim_sample(unet, x, t, clip_denoised=False, denoised_fn=denoised_fn, cond_fn=cond_fn, model_kwargs={}, eta=0.8)
 
     return step, x, ddim, (n_over + n_inner) * batches * len(names)
 
@@ -224,18 +243,19 @@ def run_reference(args, rank):
     torch.set_num_threads(os.cpu_count() or 1)
     torch.manual_seed(1234)
     step, x, ddim, cuts = build_cpu_reference(wl, world=args.gpus, scaling=args.scaling)
-    t0 = time.time()
     i = ddim - 1
-    x = step(x, i)  # warm-up (also sizes the timed part)
-    t_first = time.time() - t0
-    k = max(1, min(args.steps, int((args.cpu_budget_s - t_first) / max(t_first, 1e-3))))
+    x = step(x, i)["sample"]  # warm-up
+    k = args.steps
     t0 = time.time()
     for j in range(k):
         i = i - 1 if i > 0 else ddim - 1
-        x = step(x, i)
+        out = step(x, i)
+        x = out["sample"]
     dt = (time.time() - t0) / k
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"sample": out["sample"], "pred_xstart": out["pred_xstart"]})
     val = 1.0 / dt
-    sample = "%d full guidance step(s) after 1 warm-up step (requested %d/%d; bounded to %.0f s of CPU time)" % (k, args.steps, args.warmup, args.cpu_budget_s)
+    sample = "%d full guidance step(s) after 1 warm-up step" % k
     line = {
         "impl": "reference", "metric": METRIC % (WORKLOADS[wl][0], WORKLOADS[wl][0]), "value": cuts * val, "unit": "cutouts/s", "n_gpus": args.gpus, "steps": k,
         "warmup": 1, "ms_per_step": dt * 1e3, "higher_is_better": True, "scaling": args.scaling, "vs_baseline": None, "dtype": "f32", "data": "synthetic",
@@ -409,7 +429,8 @@ def main():
         wall0 = time.time()
         e0.record()
         for _ in range(K):
-            x = step(x, i)["sample"]
+            last = step(x, i)
+            x = last["sample"]
             i = next_i(i)
         e1.record()
         res["host_enqueue_ms"] = (time.time() - wall0) * 1e3 / K  # host time to ISSUE a step (the GPU runs behind it): the floor of the e2e step
@@ -421,6 +442,8 @@ def main():
         res["launches"] = _lib.kernel_launches - k0
         if unet_graphed:  # our GroupNorm / resample / concat kernels replayed inside the UNet's CUDA graphs (one forward + one backward per step)
             res["launches"] += K * unet.own_kernels_per_replay
+        if profile and rank == 0 and args.dump_outputs:  # the last timed step's result, copied outside the timed region
+            res["outputs"] = {"sample": last["sample"].float().cpu(), "pred_xstart": last["pred_xstart"].float().cpu()}
         if not profile:
             return res
         if clocks is not None and os.environ.get("CG_BENCH_CLOCKS_ALL_REGIONS") != "1":
@@ -460,6 +483,8 @@ def main():
         if world > 1:
             dist.destroy_process_group()
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, main_res["outputs"])
     ms, ms_e2e, cuts_per_step = main_res["ms"], main_res["ms_e2e"], main_res["cuts_per_step"]
     tf_peak, hbm_peak, peak_src = measured_peaks()
     traffic = None  # dram bytes per GEMM launch from the committed ncu capture of this same command (profiles/)

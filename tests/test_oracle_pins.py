@@ -14,7 +14,8 @@ from oracle import ref_stubs
 from oracle import resize_right as RR
 
 GOLDEN = os.path.join(os.path.dirname(__file__), "golden")
-needs_reference = pytest.mark.skipif(not ref_stubs.available(), reason="/root/reference is only present in the build container")
+needs_reference = pytest.mark.skipif(not ref_stubs.available(), reason="needs the original clip-diffusion source tree (set CLIPGUIDE_REFERENCE_ROOT); "
+                                     "test_golden_* compare with what it produced")
 
 
 def test_golden_cutouts_bit_exact():

@@ -46,7 +46,7 @@ def test_record_invariants(cfg):
     assert (rec.size, rec.x0, rec.y0, rec.flags, rec.angle, rec.perm) == (rec2.size, rec2.x0, rec2.y0, rec2.flags, rec2.angle, rec2.perm)
 
 
-@pytest.mark.skipif(not ref_stubs.available(), reason="/root/reference is only present in the build container")
+@pytest.mark.skipif(not ref_stubs.available(), reason="needs the original clip-diffusion source tree (set CLIPGUIDE_REFERENCE_ROOT)")
 @settings(max_examples=15, deadline=None)
 @given(configs)
 def test_reference_in_place_equals_oracle_for_any_configuration(cfg):

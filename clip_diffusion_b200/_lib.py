@@ -81,6 +81,9 @@ _SIGNATURES = {
     "cg_gemm_bf16_tn": (_I, [_P, _P, _I, _I, _I, _L, _L, _I, _P, _P, _P, _L, _P, _I, _P]),
     "cg_attention_fwd": (_I, [_P, _I, _I, _I, _P, _P, _P]),
     "cg_attention_bwd": (_I, [_P, _P, _P, _P, _I, _I, _I, _P, _P, _P]),
+    "cg_attention_causal_fwd": (_I, [_P, _I, _I, _I, _P, _P, _P]),
+    "cg_text_embed_fwd": (_I, [_P, _P, _P, _I, _I, _I, _I, _P, _P]),
+    "cg_text_pool_fwd": (_I, [_P, _P, _I, _I, _I, _P, _P, _P, _P]),
     "cg_vit_set_cls_rows": (_I, [_P, _P, _I, _I, _I, _P, _P]),
     "cg_vit_proj_fwd": (_I, [_P, _P, _I, _I, _I, _P, _P]),
     "cg_vit_proj_bwd": (_I, [_P, _P, _I, _I, _I, _P, _P]),

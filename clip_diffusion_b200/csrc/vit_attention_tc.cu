@@ -191,6 +191,13 @@ __device__ __forceinline__ void tmem_st32(uint32_t taddr, const uint32_t* r) {
       "r"(r[25]), "r"(r[26]), "r"(r[27]), "r"(r[28]), "r"(r[29]), "r"(r[30]), "r"(r[31])
       : "memory");
 }
+__device__ __forceinline__ void tmem_st16(uint32_t taddr, const uint32_t* r) {
+  asm volatile(
+      "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16};" ::"r"(taddr),
+      "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]), "r"(r[8]), "r"(r[9]), "r"(r[10]), "r"(r[11]), "r"(r[12]),
+      "r"(r[13]), "r"(r[14]), "r"(r[15])
+      : "memory");
+}
 __device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 
 // ---- warp-level mma.sync helpers of the edge-token path.  The edge token needs matrix-VECTOR products only (a [rows x 64] operand
@@ -401,12 +408,20 @@ __device__ __forceinline__ void fwd_edge_token_b(uint32_t sV, int Tp, float* pve
 #define TRI(slot, ev) do { } while (0)
 #endif
 
+// CAUSAL (the CLIP text transformer): column j of row i is masked (-inf) when j > i, with i = tile * 128 + row and j = block * 64 +
+// column.  Fully masked blocks are NOT skipped -- every block still runs through every role, so the barrier phases stay as described
+// above (at T = 77 such a block costs little).  A row whose share of a block is fully masked stages P = 0 for all 64 columns (a
+// select, never an exp of -inf - -inf), keeps its row sum at 0 and, if this was the warpgroup's first block of the tile, its
+// reference maximum at -inf; the next block with a kept column rescales the (zero) accumulator by ex2(-inf) = 0 like any other
+// reference move.  In the epilogue merge such a partial result weighs ex2(-inf - M) = 0, and M is finite because column 0 is kept
+// for every row, so the other warpgroup's result stands.  The edge token is off (p.edge = 0, compiled out here).
+template <bool CAUSAL>
 __global__ void __launch_bounds__(AT_THREADS, 1)
     attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_constant__ CUtensorMap tmQKVtail, const AttnParams p) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   cg_griddep_launch();
   const int T = p.T, heads = p.heads, D = heads * 64;
-  const int edge = p.edge, Tp = T - edge;  // Tp tokens go through the tensor-core pipeline; with edge = 1 token Tp is handled on CUDA cores
+  const int edge = CAUSAL ? 0 : p.edge, Tp = T - edge;  // Tp tokens go through the tensor-core pipeline; with edge = 1 token Tp is handled on CUDA cores
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int ntiles = p.ntiles, nblk = p.nblk, nblk_ld = p.nblk_ld;
   const int G = ntiles * nblk, nitems = p.nitems;
@@ -616,7 +631,15 @@ __global__ void __launch_bounds__(AT_THREADS, 1)
           TRF(warp, g, 0);
           // block maximum over the valid columns
           float bm = -INFINITY;
-          if (!tail) {
+          // causal: columns [0, lim) of this block are kept for this thread's row (lim <= 0: none)
+          const int lim = CAUSAL ? min(tail ? tail_cols : 64, tile * 128 + rl - blk * 64 + 1) : 64;
+          if constexpr (CAUSAL) {
+#pragma unroll
+            for (int j = 0; j < 32; ++j) {
+              if (j < lim) bm = fmaxf(bm, __uint_as_float(sa[j]));
+              if (32 + j < lim) bm = fmaxf(bm, __uint_as_float(sb[j]));
+            }
+          } else if (!tail) {
 #pragma unroll
             for (int j = 0; j < 32; ++j) bm = fmaxf(bm, fmaxf(__uint_as_float(sa[j]), __uint_as_float(sb[j])));
           } else {
@@ -640,13 +663,25 @@ __global__ void __launch_bounds__(AT_THREADS, 1)
               tcgen05_fence_after();
               const float f = grow ? ex2f(mref - bm) : 1.f;
               const uint32_t t_o = t_lane + 256u + (uint32_t)((2 * wg + (tile & 1)) * 64);
+              if constexpr (CAUSAL) {
+                // 16 columns at a time: lim stays live across this block, and 32 more registers next to sb would spill
 #pragma unroll
-              for (int c = 0; c < 64; c += 32) {  // (sa is dead here: it is fetched again below)
-                tmem_ld32(t_o + (uint32_t)c, sa);
-                tmem_ld_wait();
+                for (int c = 0; c < 64; c += 16) {
+                  tmem_ld16(t_o + (uint32_t)c, sa);
+                  tmem_ld_wait();
 #pragma unroll
-                for (int j = 0; j < 32; ++j) sa[j] = __float_as_uint(__uint_as_float(sa[j]) * f);
-                tmem_st32(t_o + (uint32_t)c, sa);
+                  for (int j = 0; j < 16; ++j) sa[j] = __float_as_uint(__uint_as_float(sa[j]) * f);
+                  tmem_st16(t_o + (uint32_t)c, sa);
+                }
+              } else {
+#pragma unroll
+                for (int c = 0; c < 64; c += 32) {  // (sa is dead here: it is fetched again below)
+                  tmem_ld32(t_o + (uint32_t)c, sa);
+                  tmem_ld_wait();
+#pragma unroll
+                  for (int j = 0; j < 32; ++j) sa[j] = __float_as_uint(__uint_as_float(sa[j]) * f);
+                  tmem_st32(t_o + (uint32_t)c, sa);
+                }
               }
               tmem_st_wait();
               tcgen05_fence_before();
@@ -667,7 +702,17 @@ __global__ void __launch_bounds__(AT_THREADS, 1)
             }
             const uint32_t* sv = hlf ? sb : sa;
             float a0 = 0.f, a1 = 0.f;  // independent partial sums
-            if (!tail) {
+            if constexpr (CAUSAL) {
+#pragma unroll
+              for (int j = 0; j < 16; ++j) {
+                float p0 = ex2f(fmaf(__uint_as_float(sv[2 * j]), sl2, -mref)), p1 = ex2f(fmaf(__uint_as_float(sv[2 * j + 1]), sl2, -mref));
+                if (hlf * 32 + 2 * j >= lim) p0 = 0.f;  // (also replaces the inf / NaN of a fully masked row: mref = -inf)
+                if (hlf * 32 + 2 * j + 1 >= lim) p1 = 0.f;
+                a0 += p0;
+                a1 += p1;
+                w[j] = pack_bf2(p0, p1);
+              }
+            } else if (!tail) {
 #pragma unroll
               for (int j = 0; j < 16; ++j) {
                 const float p0 = ex2f(fmaf(__uint_as_float(sv[2 * j]), sl2, -mref)), p1 = ex2f(fmaf(__uint_as_float(sv[2 * j + 1]), sl2, -mref));
@@ -1437,17 +1482,14 @@ int launch_attn_bwd_tc(const void* qkv, const void* dctx, int Nimg, int T, int h
   return 0;
 }
 
-}  // namespace
-
-// Return 0 when the tcgen05 path handled the call, 1 when the caller should use the mma.sync kernel (T > 272 or CG_ATTN_TC=0), or an error.
-int cg_attention_fwd_tc(const void* qkv, int Nimg, int T, int heads, void* ctx, float* lse, cudaStream_t s) {
-  if (T > 272 || !tc_enabled()) return 1;
+template <bool CAUSAL>
+int launch_attn_fwd_tc(const void* qkv, int Nimg, int T, int heads, void* ctx, float* lse, bool allow_edge, cudaStream_t s) {
   AttnParams p = {};
   p.ctx = reinterpret_cast<__nv_bfloat16*>(ctx);
   p.lse = lse;
   p.T = T; p.heads = heads; p.scale = 0.125f;
   p.trace = g_trace;
-  set_geometry(p, T, fwd_edge_enabled());
+  set_geometry(p, T, allow_edge);
   const int D = heads * 64;
   CUtensorMap tq, tqt;
   int rc = cg_make_tensor_map_bf16(&tq, qkv, (long long)Nimg * T, 3LL * D, 3LL * D, 64);
@@ -1460,12 +1502,27 @@ int cg_attention_fwd_tc(const void* qkv, int Nimg, int T, int heads, void* ctx, 
   const int grid = p.nitems < cg_num_sms() ? p.nitems : cg_num_sms();  // persistent: one CTA per SM
   static size_t configured[CG_MAX_DEVICES] = {};
   const int dev = cg_device_index();
-  if (smem > configured[dev]) {
-    CG_CUDA(cudaFuncSetAttribute(attn_fwd_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  if (smem > configured[dev]) {  // (one cache per instantiation: function attributes are per kernel)
+    CG_CUDA(cudaFuncSetAttribute(attn_fwd_tc_kernel<CAUSAL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     configured[dev] = smem;
   }
-  CG_CUDA(cg_launch_pdl(attn_fwd_tc_kernel, dim3(grid), dim3(AT_THREADS), smem, s, tq, tqt, p));
+  CG_CUDA(cg_launch_pdl(attn_fwd_tc_kernel<CAUSAL>, dim3(grid), dim3(AT_THREADS), smem, s, tq, tqt, p));
   return 0;
+}
+
+}  // namespace
+
+// Return 0 when the tcgen05 path handled the call, 1 when the caller should use the mma.sync kernel (T > 272 or CG_ATTN_TC=0), or an error.
+int cg_attention_fwd_tc(const void* qkv, int Nimg, int T, int heads, void* ctx, float* lse, cudaStream_t s) {
+  if (T > 272 || !tc_enabled()) return 1;
+  return launch_attn_fwd_tc<false>(qkv, Nimg, T, heads, ctx, lse, fwd_edge_enabled(), s);
+}
+
+// The CLIP text transformer's attention (OpenAI encode_text, utils/functional.py:91-94): tcgen05 path only, no edge token.
+extern "C" int cg_attention_causal_fwd(const void* qkv, int Nseq, int T, int heads, void* ctx, float* lse, void* stream) {
+  CG_REQUIRE(qkv && ctx && lse && Nseq > 0 && T > 0 && heads > 0, "cg_attention_causal_fwd: bad arguments");
+  CG_REQUIRE(T <= 272, "cg_attention_causal_fwd: T=%d exceeds the tcgen05 kernel's limit (272)", T);
+  return launch_attn_fwd_tc<true>(qkv, Nseq, T, heads, ctx, lse, false, cg_stream(stream));
 }
 
 int cg_attention_bwd_tc(const void* qkv, const void* ctx, const void* dctx, const float* lse, int Nimg, int T, int heads, void* dqkv, cudaStream_t s) {

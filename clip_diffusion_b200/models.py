@@ -1,4 +1,4 @@
-"""CLIP image towers for the guidance path, B200-native (mirror of clip_diffusion/models.py:33-84,188-240).
+"""CLIP towers for the guidance path, B200-native (mirror of clip_diffusion/models.py:33-84,188-240).
 
 ``load_clip_models(names, device)`` returns ``{name: model}`` where ``model`` exposes what the hot path
 touches on an OpenAI ``clip`` model: ``model.visual.input_resolution`` (sample.py:167) and
@@ -11,6 +11,9 @@ reference gets from the un-vendored ``clip`` package -- is implemented here on t
   attention              fused kernels (scores never leave the SM)
   backward               dgrad only: the towers are frozen (models.py:67-71), so every backward GEMM is
                          activation-gradient x pre-transposed weight, packed once at load
+
+``model.encode_text(tokens)`` (utils/functional.py:91-94, once per job) runs OpenAI's text transformer on the same kernels with
+a causal attention forward; that tower is built on its first call.
 
 There is no network here, so weights are constructor-style random init (SURVEY.md App. A.1) unless a
 state dict in OpenAI's key naming is supplied.
@@ -34,11 +37,27 @@ CLIP_CONFIGS = {
 _CLIP_DIMS = {"ViT-B/32": 512, "ViT-B/16": 512, "ViT-L/14": 768, "ViT-L/14@336px": 768}
 
 
+# name: (context_length, vocab_size, width, layers, heads, embed_dim) of the text transformer (OpenAI clip/model.py build_model)
+CLIP_TEXT_CONFIGS = {
+    "ViT-B/32": (77, 49408, 512, 12, 8, 512),
+    "ViT-B/16": (77, 49408, 512, 12, 8, 512),
+    "ViT-L/14": (77, 49408, 768, 12, 12, 768),
+    "ViT-L/14@336px": (77, 49408, 768, 12, 12, 768),
+}
+
+
 def register_clip_config(name, input_resolution, patch, width, layers, heads, embed_dim):
     """Extra tower shapes (tests use tiny ones).  width must be heads*64 and a multiple of 128."""
     if width != heads * 64 or width % 128:
         raise ValueError("width must equal heads*64 and be a multiple of 128")
     CLIP_CONFIGS[name] = (input_resolution, patch, width, layers, heads, embed_dim)
+
+
+def register_clip_text_config(name, context, vocab, width, layers, heads, embed_dim):
+    """Extra text-tower shapes (tests use tiny ones), same constraints as register_clip_config; context <= 272."""
+    if width != heads * 64 or width % 128 or not 0 < context <= 272:
+        raise ValueError("width must equal heads*64 and be a multiple of 128, and the context length at most 272")
+    CLIP_TEXT_CONFIGS[name] = (context, vocab, width, layers, heads, embed_dim)
 
 
 def random_clip_state_dict(name, seed=1):
@@ -71,6 +90,56 @@ def random_clip_state_dict(name, seed=1):
         for ln in ("ln_1", "ln_2"):
             sd[p + ln + ".weight"] = 1 + 0.1 * n(width)
             sd[p + ln + ".bias"] = 0.1 * n(width)
+    return sd
+
+
+def clip_text_state_dict_keys(name):
+    """The text-tower keys of an OpenAI CLIP state dict (everything encode_text reads), in OpenAI's naming."""
+    layers = CLIP_TEXT_CONFIGS[name][3]
+    keys = ["token_embedding.weight", "positional_embedding"]
+    for i in range(layers):
+        p = "transformer.resblocks.%d." % i
+        keys += [p + k for k in ("attn.in_proj_weight", "attn.in_proj_bias", "attn.out_proj.weight", "attn.out_proj.bias", "mlp.c_fc.weight",
+                                 "mlp.c_fc.bias", "mlp.c_proj.weight", "mlp.c_proj.bias", "ln_1.weight", "ln_1.bias", "ln_2.weight", "ln_2.bias")]
+    return keys + ["ln_final.weight", "ln_final.bias", "text_projection"]
+
+
+def clip_text_state_dict_shapes(name):
+    """{key: shape} of the text tower from CLIP_TEXT_CONFIGS, in the order of clip_text_state_dict_keys."""
+    context, vocab, width, layers, heads, embed = CLIP_TEXT_CONFIGS[name]
+    known = {"token_embedding.weight": (vocab, width), "positional_embedding": (context, width), "text_projection": (width, embed),
+             "attn.in_proj_weight": (3 * width, width), "attn.in_proj_bias": (3 * width,), "attn.out_proj.weight": (width, width),
+             "mlp.c_fc.weight": (4 * width, width), "mlp.c_fc.bias": (4 * width,), "mlp.c_proj.weight": (width, 4 * width)}
+    # block keys are looked up by their leaf ("transformer.resblocks.<i>.<leaf>"); every other tensor is [width]
+    return {k: known.get(k.split(".", 3)[-1] if k.startswith("transformer.") else k, (width,)) for k in clip_text_state_dict_keys(name)}
+
+
+def random_clip_text_state_dict(name, seed=1):
+    """Random weights with the keys and shapes of OpenAI's text tower.  Standard deviations follow OpenAI's
+    ``CLIP.initialize_parameters`` (token 0.02, positional 0.01, attention width^-0.5, out / c_proj width^-0.5 (2 layers)^-0.5,
+    c_fc (2 width)^-0.5, projection width^-0.5); LayerNorm affines and biases are perturbed as in random_clip_state_dict."""
+    context, vocab, width, layers, heads, embed = CLIP_TEXT_CONFIGS[name]
+    g = torch.Generator().manual_seed(seed)
+    u = lambda *s, fan: (torch.rand(*s, generator=g) * 2 - 1) / math.sqrt(fan)
+    n = lambda *s: torch.randn(*s, generator=g)
+    attn_std, proj_std, fc_std = width ** -0.5, width ** -0.5 * (2 * layers) ** -0.5, (2 * width) ** -0.5
+    sd = {"token_embedding.weight": 0.02 * n(vocab, width), "positional_embedding": 0.01 * n(context, width)}
+    for i in range(layers):
+        p = "transformer.resblocks.%d." % i
+        sd[p + "attn.in_proj_weight"] = attn_std * n(3 * width, width)
+        sd[p + "attn.in_proj_bias"] = 0.02 * n(3 * width)
+        sd[p + "attn.out_proj.weight"] = proj_std * n(width, width)
+        sd[p + "attn.out_proj.bias"] = 0.02 * n(width)
+        sd[p + "mlp.c_fc.weight"] = fc_std * n(4 * width, width)
+        sd[p + "mlp.c_fc.bias"] = u(4 * width, fan=width)
+        sd[p + "mlp.c_proj.weight"] = proj_std * n(width, 4 * width)
+        sd[p + "mlp.c_proj.bias"] = u(width, fan=4 * width)
+        for ln in ("ln_1", "ln_2"):
+            sd[p + ln + ".weight"] = 1 + 0.1 * n(width)
+            sd[p + ln + ".bias"] = 0.1 * n(width)
+    sd["ln_final.weight"] = 1 + 0.1 * n(width)
+    sd["ln_final.bias"] = 0.1 * n(width)
+    sd["text_projection"] = width ** -0.5 * n(width, embed)
     return sd
 
 
@@ -285,6 +354,72 @@ class VisionTransformerB200:
         return n * (fwd + bwd)
 
 
+class TextTransformerB200:
+    """Frozen OpenAI CLIP text transformer (``CLIP.encode_text``), forward only, on sm_100a kernels.  It runs once per job
+    (preprocessing.py:11-24), so every pass is eager with per-call activation buffers: no CUDA graphs, no workspace cache."""
+
+    def __init__(self, name, state_dict, device):
+        context, vocab, width, layers, heads, embed = CLIP_TEXT_CONFIGS[name]
+        self.name = name
+        self.context_length, self.vocab_size, self.width, self.layers, self.heads, self.output_dim = context, vocab, width, layers, heads, embed
+        self.device = torch.device(device)
+        sd, dev = state_dict, self.device
+        self.token_embedding = _f32(sd["token_embedding.weight"], dev)
+        self.pos = _f32(sd["positional_embedding"], dev)
+        self.ln_final = (_f32(sd["ln_final.weight"], dev), _f32(sd["ln_final.bias"], dev))
+        self.proj = _f32(sd["text_projection"], dev)
+        self.blocks = []
+        for i in range(layers):
+            p = "transformer.resblocks.%d." % i
+            blk = {
+                "ln1": (_f32(sd[p + "ln_1.weight"], dev), _f32(sd[p + "ln_1.bias"], dev)),
+                "ln2": (_f32(sd[p + "ln_2.weight"], dev), _f32(sd[p + "ln_2.bias"], dev)),
+            }
+            # W [N, K] bf16 as the GEMM's B operand; no transposed copies (no dgrad)
+            for key, src in (("qkv", "attn.in_proj_weight"), ("out", "attn.out_proj.weight"), ("fc", "mlp.c_fc.weight"), ("proj", "mlp.c_proj.weight")):
+                blk["w_" + key] = _bf16(sd[p + src], dev)
+            blk["b_qkv"] = _f32(sd[p + "attn.in_proj_bias"], dev)
+            blk["b_out"] = _f32(sd[p + "attn.out_proj.bias"], dev)
+            blk["b_fc"] = _f32(sd[p + "mlp.c_fc.bias"], dev)
+            blk["b_proj"] = _f32(sd[p + "mlp.c_proj.bias"], dev)
+            self.blocks.append(blk)
+
+    def forward_tokens(self, tokens):
+        """tokens: int32 [N, context] on the tower's device, ids in [0, vocab) -> embeddings [N, E] fp32."""
+        n, T, D, E = tokens.shape[0], self.context_length, self.width, self.output_dim
+        M = n * T
+        dev = self.device
+        f32 = lambda *s: torch.empty(*s, device=dev, dtype=torch.float32)
+        b16 = lambda *s: torch.empty(*s, device=dev, dtype=torch.bfloat16)
+        x, x_mid, mean, rstd = f32(M, D), f32(M, D), f32(M), f32(M)
+        h, qkv, ctx, hg, u, lse = b16(M, D), b16(M, 3 * D), b16(M, D), b16(M, 4 * D), b16(M, 4 * D), f32(n, self.heads, T)
+        y, emb = f32(n, D), f32(n, E)
+        P, C = _lib.ptr, _lib.call
+        C("cg_text_embed_fwd", P(tokens), P(self.token_embedding), P(self.pos), n, T, D, self.vocab_size, P(x))
+        for blk in self.blocks:
+            C("cg_layernorm_fwd", P(x), P(blk["ln1"][0]), P(blk["ln1"][1]), M, D, D, P(h), None, P(mean), P(rstd))
+            gemm_bf16_tn(h, blk["w_qkv"], _lib.EPI_BIAS_BF16, bias=blk["b_qkv"], out=qkv)
+            C("cg_attention_causal_fwd", P(qkv), n, T, self.heads, P(ctx), P(lse))
+            gemm_bf16_tn(ctx, blk["w_out"], _lib.EPI_BIAS_RESID_F32, bias=blk["b_out"], out=x_mid, aux=x)
+            C("cg_layernorm_fwd", P(x_mid), P(blk["ln2"][0]), P(blk["ln2"][1]), M, D, D, P(h), None, P(mean), P(rstd))
+            gemm_bf16_tn(h, blk["w_fc"], _lib.EPI_BIAS_QGELU_BF16, bias=blk["b_fc"], out=hg, aux=u)  # (u: the pre-activation, unused)
+            gemm_bf16_tn(hg, blk["w_proj"], _lib.EPI_BIAS_RESID_F32, bias=blk["b_proj"], out=x, aux=x_mid)
+        C("cg_text_pool_fwd", P(x), P(tokens), n, T, D, P(self.ln_final[0]), P(self.ln_final[1]), P(y))
+        C("cg_vit_proj_fwd", P(y), P(self.proj), n, D, E, P(emb))
+        return emb
+
+
+def _check_text_state_dict(name, sd, where):
+    """KeyError naming the first missing text-tower key, ValueError on a shape that does not match CLIP_TEXT_CONFIGS (host only)."""
+    shapes = clip_text_state_dict_shapes(name)
+    missing = [k for k in shapes if k not in sd]
+    if missing:
+        raise KeyError("%s lacks %d text-tower keys (first: %s): expected OpenAI CLIP naming" % (where, len(missing), missing[0]))
+    for k, shape in shapes.items():
+        if tuple(sd[k].shape) != shape:
+            raise ValueError("%s: %s has shape %s, the %s text tower needs %s" % (where, k, tuple(sd[k].shape), name, shape))
+
+
 class _EncodeImageFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, image, tower, normalize):
@@ -331,6 +466,10 @@ class CLIPModelB200:
         self.name = name
         sd = state_dict if state_dict is not None else random_clip_state_dict(name, seed)
         self.visual = _Visual(VisionTransformerB200(name, sd, device))
+        # the text tower is built on the first encode_text (image-only use keeps its memory and load time): until then the
+        # checkpoint's non-visual tensors stay where the caller put them (load_clip_models: host memory); random init is seeded
+        self._seed, self._text = seed, None
+        self._text_sd = None if state_dict is None else {k: v for k, v in state_dict.items() if not k.startswith("visual.")}
 
     def encode_image(self, image):
         """image: CLIP-normalised [N,3,res,res] -> [N,E] fp32 (differentiable w.r.t. image)."""
@@ -341,7 +480,33 @@ class CLIPModelB200:
         return _EncodeImageFn.apply(image01, self.visual.tower, True)
 
     def encode_text(self, text):
-        raise NotImplementedError("the text tower runs once per job (preprocessing.py:11-24) and is not part of the guidance hot path")
+        """OpenAI ``CLIP.encode_text``: token ids [N, context] (int32 or int64, as ``clip.tokenize(...).to(device)`` gives them) ->
+        [N, E] fp32 without grad_fn.  The sequence is pooled at its first maximal id (the end-of-text token)."""
+        if self.name not in CLIP_TEXT_CONFIGS:
+            raise ValueError("no text-tower configuration for %r (CLIP_TEXT_CONFIGS)" % self.name)
+        context, vocab = CLIP_TEXT_CONFIGS[self.name][:2]
+        if not isinstance(text, torch.Tensor) or text.dim() != 2 or text.shape[1] != context:
+            raise ValueError("expected token ids of shape [N, %d], got %s" % (context, tuple(getattr(text, "shape", ()))))
+        if text.dtype.is_floating_point or text.dtype.is_complex or text.dtype == torch.bool:
+            raise ValueError("expected integer token ids, got %s" % text.dtype)
+        if text.shape[0] == 0:
+            raise ValueError("expected at least one sequence")
+        lo, hi = torch.stack([text.min(), text.max()]).tolist()  # the one host read of the call
+        if lo < 0 or hi >= vocab:
+            raise ValueError("token ids must lie in [0, %d), got [%d, %d]" % (vocab, lo, hi))
+        sd = None
+        if self._text is None:
+            sd = self._text_sd if self._text_sd is not None else random_clip_text_state_dict(self.name, self._seed)
+            _check_text_state_dict(self.name, sd, "the %s checkpoint" % self.name)
+        _lib.require_cuda(text)
+        model_device = self.visual.tower.pos.device  # (an explicit index, unlike a bare "cuda")
+        if text.device != model_device:
+            raise ValueError("token ids are on %s, the model on %s" % (text.device, model_device))
+        if self._text is None:
+            self._text = TextTransformerB200(self.name, sd, model_device)
+            self._text_sd = None
+        with torch.no_grad():
+            return self._text.forward_tokens(text.to(torch.int32).contiguous())
 
     def eval(self):
         return self
@@ -357,7 +522,9 @@ def load_clip_models(model_names, device=None, allow_random_init=False):
     """models.py:74-84.  Weights: ``$CLIPGUIDE_B200_WEIGHTS/<name with / -> _>.pt``, a state dict in OpenAI's key naming
     (``visual.conv1.weight`` ...; what ``clip.load(name).state_dict()`` holds).  A missing directory or file is an ERROR --
     guidance with random weights is meaningless -- unless the caller opts in with ``allow_random_init=True`` (benchmarks and
-    tests: there is no network on the benchmark boxes, and throughput does not depend on the weight values)."""
+    tests: there is no network on the benchmark boxes, and throughput does not depend on the weight values).  Only the
+    ``visual.*`` keys are checked here; the text tower's tensors (``token_embedding.weight`` ...) stay in host memory until the
+    first ``encode_text``, which checks and uploads them (a visual-only checkpoint loads; its encode_text raises KeyError)."""
     device = device or "cuda"
     wdir = os.environ.get("CLIPGUIDE_B200_WEIGHTS")
     models = {}

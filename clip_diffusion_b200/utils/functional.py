@@ -36,7 +36,8 @@ def embed_image(clip_model, image, clip_normalize=True, L2_normalize=False):
 
 
 def embed_text(clip_model, text, L2_normalize=False):
-    """functional.py:91-94 (runs once per job; the B200 models raise: text towers are outside this path)"""
+    """functional.py:91-94: token ids [P, 77] (clip.tokenize output on the model's device) -> [P, E] fp32.  Runs once per job
+    (preprocessing.py:11-24); the B200 models encode on the sm_100a kernels (CLIPModelB200.encode_text), without autograd."""
     text_embedding = clip_model.encode_text(text).float()
     return text_embedding if not L2_normalize else L2_norm(text_embedding, dim=-1)
 

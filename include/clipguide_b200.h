@@ -196,6 +196,21 @@ int cg_vit_tokens_to_bf16(const float* x, int Nimg, int T, int D, int drop_cls, 
 int cg_patchify_fwd(const float* img, int N, int cs, int patch, int kpad, int normalize, void* out_bf16, void* stream);
 int cg_patchify_bwd(const void* dpatch, int dpatch_is_f32, int N, int cs, int patch, int kpad, int normalize, float* dimg, void* stream);
 
+/* The OpenAI CLIP text transformer (CLIP.encode_text, reached through embed_text, utils/functional.py:91-94; the reference encodes
+ * its prompts with it once per job, preprocessing.py:11-24).  Forward only: the text side is a constant of the guidance step.
+ *   x = token_embedding[tokens] + positional_embedding;  L x {x += MHA_causal(ln_1 x); x += c_proj(QuickGELU(c_fc(ln_2 x)))};
+ *   out = ln_final(x)[n, argmax_t tokens[n, t]] @ text_projection
+ * The blocks use cg_layernorm_fwd, cg_gemm_bf16_tn and the causal attention below; the projection is cg_vit_proj_fwd. */
+/* cg_attention_fwd with a causal mask (key j > query i is -inf): same layout, scale and outputs; lse [Nseq, heads, T] is the
+ * log-sum-exp over the keys j <= i.  tcgen05 kernel only: T <= 272 (CG_EINVAL beyond; OpenAI's context length is 77). */
+int cg_attention_causal_fwd(const void* qkv, int Nseq, int T, int heads, void* ctx, float* lse, void* stream);
+/* x[n*T + t, :] = token_embedding[tokens[n, t], :] + pos[t, :].  tokens [N, T] int32, token_embedding [V, D] fp32, pos [T, D] fp32,
+ * x [N*T, D] fp32 (residual stream); D % 4 == 0.  The table is never read outside [0, V): a row whose id lies outside gets NaN. */
+int cg_text_embed_fwd(const int* tokens, const float* token_embedding, const float* pos, int N, int T, int D, int V, float* x, void* stream);
+/* End-of-text pooling + ln_final: e_n = the first t with tokens[n, t] maximal (torch.argmax; the end-of-text id 49407 is the largest),
+ * y[n, :] = LayerNorm(x[n*T + e_n, :]) * gamma + beta (eps 1e-5).  x [N*T, D], y [N, D] fp32; D % 4 == 0. */
+int cg_text_pool_fwd(const float* x, const int* tokens, int N, int T, int D, const float* gamma, const float* beta, float* y, void* stream);
+
 /* ------------------------------------------------------------------ cond_fn tail ---------- */
 /* sample.py:228-238: NaN guard + RMS-normalised clamp, on device (no host sync):
  *   if (bad) out = 0 else { m = sqrt(mean(g^2)); out = sign * g * clamp(m,-thr,thr)/m }

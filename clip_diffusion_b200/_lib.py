@@ -110,6 +110,9 @@ launch_count = 0     # C-ABI calls made through this module
 kernel_launches = 0  # CUDA kernels those calls launched (bench.py reports it as gpu_launches)
 # kernels launched per entry point (csrc/*.cu); 1 unless listed
 _KERNELS_PER_CALL = {"cg_cutouts_fwd": 4, "cg_cutouts_bwd": 4, "cg_ms_ssim_dissimilarity_fwd_bwd": 17, "cg_attention_bwd": 3, "cg_grad_finalize": 2, "cg_any_nan": 2, "cg_dynamic_threshold": 5, "cg_groupnorm_nhwc_fwd": 3, "cg_groupnorm_nhwc_bwd": 3}
+# longest sequence of the tcgen05 attention kernels (ATTN_TC_MAX_T in csrc/tcgen05.cuh); cg_attention_fwd / _bwd run longer ones
+# on the mma.sync kernels, and cg_attention_causal_fwd refuses them
+ATTN_TC_MAX_T = 272
 
 
 class ClipGuideError(RuntimeError):
@@ -183,7 +186,7 @@ def call(name, *args):
         ev1.record()
         PROFILE.append((name, args, ev0, ev1))
     launch_count += 1
-    if name == "cg_attention_bwd" and args[5] <= 272 and os.environ.get("CG_ATTN_TC", "1") != "0":
+    if name == "cg_attention_bwd" and args[5] <= ATTN_TC_MAX_T:
         kernel_launches += 1  # one persistent tcgen05 kernel (delta included); the mma.sync path beyond T = 272 is delta + dQ + dK/dV
     else:
         kernel_launches += _KERNELS_PER_CALL.get(name, 1)

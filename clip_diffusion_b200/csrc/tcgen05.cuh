@@ -91,3 +91,11 @@ __device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.p
 // host: cached cuTensorMapEncodeTiled for a [rows, cols] bf16 row-major matrix (leading dimension ld elements), box = 64
 // columns x box_rows rows, 128-byte swizzle (defined in vit_gemm.cu)
 int cg_make_tensor_map_bf16(CUtensorMap* out, const void* ptr, long long rows, long long cols, long long ld, int box_rows);
+// host: multiprocessor count of the current device, cached per device (defined in vit_gemm.cu); sizes the persistent grids
+int cg_num_sms();
+
+// host: the tcgen05 attention kernels (vit_attention_tc.cu) keep all operands of an (image, head) item in shared memory, which holds
+// sequences up to this length; cg_attention_fwd / _bwd run longer ones on the mma.sync kernels of vit_attention.cu
+constexpr int ATTN_TC_MAX_T = 272;
+int cg_attention_fwd_tc(const void* qkv, int Nimg, int T, int heads, void* ctx, float* lse, cudaStream_t s);
+int cg_attention_bwd_tc(const void* qkv, const void* ctx, const void* dctx, const float* lse, int Nimg, int T, int heads, void* dqkv, cudaStream_t s);

@@ -1,5 +1,6 @@
-// Fused multi-head self-attention of the CLIP ViT (head_dim 64, T in {50,197,257,577}: short sequences, many
-// (cutout, head) problems), forward and dgrad.  Scores never touch HBM.
+// Fused multi-head self-attention of the CLIP ViT (head_dim 64, many (cutout, head) problems), forward and dgrad, for the
+// sequences too long for the tcgen05 kernels of vit_attention_tc.cu (T > ATTN_TC_MAX_T: ViT-L/14@336, T = 577); the entry
+// points below choose between the two from T.  Scores never touch HBM.
 //
 // Layout: packed qkv [Nimg*T, 3*D] bf16 (q | k | v; head h = columns h*64..h*64+63 of each third).
 // One CTA = one (image, head): the whole K/V (forward, dQ) or Q/dO (dK/dV) of that head is loaded into shared
@@ -12,6 +13,7 @@
 // backward = delta kernel (rowsum dO*O) + dQ kernel (per query block) + dK/dV kernel (per key block): P is
 // recomputed from q, k and the saved log-sum-exp; no atomics, deterministic.
 #include "common.cuh"
+#include "tcgen05.cuh"
 
 namespace {
 
@@ -426,17 +428,10 @@ static int pick_warps(int T) {
   return best;
 }
 
-// vit_attention_tc.cu: tcgen05/TMEM kernels for T <= 272; return 1 when they do not apply
-int cg_attention_fwd_tc(const void* qkv, int Nimg, int T, int heads, void* ctx, float* lse, cudaStream_t s);
-int cg_attention_bwd_tc(const void* qkv, const void* ctx, const void* dctx, const float* lse, int Nimg, int T, int heads, void* dqkv, cudaStream_t s);
-
 extern "C" int cg_attention_fwd(const void* qkv, int Nimg, int T, int heads, void* ctx, float* lse, void* stream) {
   CG_REQUIRE(qkv && ctx && lse && Nimg > 0 && T > 0 && heads > 0, "cg_attention_fwd: bad arguments");
-  {
-    // tcgen05/TMEM path for T <= 272 (all 224-pixel towers, the default); returns 1 when it does not apply (T too long or CG_ATTN_TC=0)
-    const int rc_tc = cg_attention_fwd_tc(qkv, Nimg, T, heads, ctx, lse, cg_stream(stream));
-    if (rc_tc != 1) return rc_tc;
-  }
+  // the tcgen05/TMEM kernels (vit_attention_tc.cu) take every sequence that fits them: all 224-pixel towers
+  if (T <= ATTN_TC_MAX_T) return cg_attention_fwd_tc(qkv, Nimg, T, heads, ctx, lse, cg_stream(stream));
   const int Tp = (T + 63) & ~63;
   CG_REQUIRE(Tp <= 640, "cg_attention_fwd: T=%d exceeds the shared-memory resident limit (640)", T);
   const int W = pick_warps(T);
@@ -456,11 +451,8 @@ extern "C" int cg_attention_bwd(const void* qkv, const void* ctx, const void* dc
   const int Tp = (T + 63) & ~63;
   CG_REQUIRE(Tp <= 640, "cg_attention_bwd: T=%d exceeds the shared-memory resident limit (640)", T);
   cudaStream_t s = cg_stream(stream);
-  {
-    // tcgen05/TMEM path (T <= 272): computes delta = rowsum(dO * O) itself (its epilogue warps, one item ahead)
-    const int rc_tc = cg_attention_bwd_tc(qkv, ctx, dctx, lse, Nimg, T, heads, dqkv, s);
-    if (rc_tc != 1) return rc_tc;
-  }
+  // the tcgen05 kernel computes delta = rowsum(dO * O) itself (its epilogue warps, one item ahead)
+  if (T <= ATTN_TC_MAX_T) return cg_attention_bwd_tc(qkv, ctx, dctx, lse, Nimg, T, heads, dqkv, s);
   const long long rows = (long long)Nimg * T;
   CG_CUDA(cg_launch_pdl(attn_delta_kernel, dim3((unsigned)((rows + 7) / 8)), dim3(256), 0, s, reinterpret_cast<const __nv_bfloat16*>(ctx),
                         reinterpret_cast<const __nv_bfloat16*>(dctx), T, heads, rows, delta_ws));

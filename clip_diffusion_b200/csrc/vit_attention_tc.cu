@@ -1,5 +1,6 @@
 // Fused multi-head self-attention of the CLIP ViT on the 5th-gen tensor cores (tcgen05 + TMEM + TMA), forward AND
-// backward, for the short sequences of the 224-pixel towers (T <= 272: ViT-B/32 T=50, ViT-B/16 T=197, ViT-L/14 T=257).
+// backward, for the short sequences of the 224-pixel towers (T <= ATTN_TC_MAX_T = 272: ViT-B/32 T=50, ViT-B/16 T=197, ViT-L/14
+// T=257); cg_attention_fwd / _bwd (vit_attention.cu) run every such T here.  The causal forward is the text transformer's attention.
 // Replaces nn.MultiheadAttention inside clip_model.encode_image (clip_diffusion/utils/functional.py:97-102) and its
 // autograd backward (sample.py:199-214).  Scores never leave the SM.
 //
@@ -27,10 +28,11 @@
 //             P is recomputed from the saved log-sum-exp; two orientations instead of a transposed smem operand, no atomics,
 //             deterministic.  Rows / columns beyond T are masked (tail block only) or never stored.
 //
-// Edge token.  T = 64 m + 1 (ViT-L/14: 16 x 16 patches + class token = 257) would leave the pipeline with a 1-row tile and a 1-column
-// block per tile, each costing a full S -> softmax -> MMA round trip (25-30% of an item).  The LAST token is therefore kept out of
-// the pipeline, which then sees only full tiles and blocks: its row and column of the score matrix are matrix-vector products, done by
-// the epilogue warps with warp-level m16n8k16 MMAs on the TMA-written tiles (ldmatrix), and folded in when a tile is written
+// Edge token (non-causal kernels).  T = 64 m + 1 (ViT-L/14: 16 x 16 patches + class token = 257) would leave the pipeline with a
+// 1-row tile and a 1-column block per tile, each costing a full S -> softmax -> MMA round trip (25-30% of an item).  The LAST token
+// is therefore kept out of the pipeline, which then sees only full tiles and blocks: its row and column of the score matrix are
+// matrix-vector products, done by the epilogue warps with warp-level m16n8k16 MMAs on the TMA-written tiles (ldmatrix), and folded
+// in when a tile is written
 // (forward: a third partial result of the online-softmax merge; backward: rank-1 corrections dQ_i += dS_ie K_e, dK_j += dS_ej Q_e,
 // dV_j += p_ej dO_e, plus the three reductions that give row e of dQ, dK, dV).
 //
@@ -46,7 +48,6 @@
 // cycles per item and warpgroup in the forward; the forward's epilogue warps (tile merges + ~9000 cycles of edge work per item) are
 // its critical resource; the backward pays ~4000 cycles per item for the single-buffered operand reload (220 KB of shared memory
 // are in use).  Under load the GPU runs these kernels at 1.45-1.8 GHz (sw_power_cap), not at 1.965.
-#include <stdlib.h>
 #include "common.cuh"
 #include "tcgen05.cuh"
 
@@ -55,7 +56,8 @@ using namespace tc;
 namespace {
 
 constexpr int AT_THREADS = 512;
-constexpr int MAX_BLK = 5;  // 64-row blocks per operand: T <= 272 -> <= 5
+constexpr int MAX_BLK = 5;  // 64-row blocks per operand
+static_assert((ATTN_TC_MAX_T + 63) / 64 <= MAX_BLK, "operand blocks of the longest sequence");
 constexpr float LOG2E_F = 1.4426950408889634f;
 constexpr uint32_t BLK_BYTES = 64 * 128;     // one 64-row operand block
 constexpr uint32_t TILE_BYTES = 128 * 128;   // one 128-row tile of an operand = one [128 x 64] staging tile
@@ -1411,20 +1413,12 @@ __global__ void __launch_bounds__(AT_THREADS, 1)
 
 long long* g_trace = nullptr;
 
-// Pipeline / load geometry.  T = 64 m + 1 (ViT-L/14: 16 x 16 patches + class token = 257): the LAST token is taken out of the tensor-core pipeline ("edge"), which then sees only full 64-wide blocks and full 128-row
-// tiles; CG_ATTN_EDGE=0 keeps it in (A/B measurements, and the narrow-tile code paths stay tested).
-int edge_env() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("CG_ATTN_EDGE");
-    v = e ? atoi(e) : 3;  // bit 0: forward, bit 1: backward
-  }
-  return v;
-}
-bool fwd_edge_enabled() { return (edge_env() & 1) != 0; }
-bool bwd_edge_enabled() { return (edge_env() & 2) != 0; }
-void set_geometry(AttnParams& p, int T, bool allow_edge) {
-  p.edge = (allow_edge && T > 1 && (T - 1) % 64 == 0) ? 1 : 0;
+// Parameters and pipeline / load geometry of one launch.  T = 64 m + 1 (ViT-L/14: 16 x 16 patches + class token = 257): the non-causal
+// kernels take the LAST token out of the tensor-core pipeline ("edge"), which then sees only full 64-wide blocks and full 128-row tiles.
+void set_geometry(AttnParams& p, int T, int heads, bool causal) {
+  p.T = T; p.heads = heads; p.scale = 0.125f;
+  p.trace = g_trace;
+  p.edge = (!causal && T > 1 && (T - 1) % 64 == 0) ? 1 : 0;
   const int Tp = T - p.edge;
   p.ntiles = (Tp + 127) / 128;
   p.nblk = (Tp + 63) / 64;
@@ -1433,106 +1427,68 @@ void set_geometry(AttnParams& p, int T, bool allow_edge) {
   p.ld_tail = p.edge ? 16 : p.tail_rows;
 }
 
-int cg_num_sms() {
-  static int per_device[CG_MAX_DEVICES] = {};
-  const int dev = cg_device_index();
-  if (per_device[dev] == 0) {
-    int n = 0;
-    cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev);
-    per_device[dev] = n > 0 ? n : CG_NUM_SMS;
-  }
-  return per_device[dev];
+// TMA maps of a [rows, cols] bf16 operand: one for its full 64-row blocks, one for the last block loaded (ld_tail rows)
+int make_operand_maps(CUtensorMap& full, CUtensorMap& tail, const void* ptr, long long rows, long long cols, const AttnParams& p) {
+  const int rc = cg_make_tensor_map_bf16(&full, ptr, rows, cols, cols, 64);
+  return rc ? rc : cg_make_tensor_map_bf16(&tail, ptr, rows, cols, cols, p.ld_tail);
 }
 
-int tc_enabled() {
-  static int enabled = -1;
-  if (enabled < 0) {
-    const char* e = getenv("CG_ATTN_TC");
-    enabled = e ? (atoi(e) != 0) : 1;  // default ON; CG_ATTN_TC=0 selects the mma.sync kernels of vit_attention.cu (A/B comparisons)
-  }
-  return enabled;
-}
-
-int launch_attn_bwd_tc(const void* qkv, const void* dctx, int Nimg, int T, int heads, const AttnParams& p0, cudaStream_t s) {
-  AttnParams p = p0;
-  p.T = T; p.heads = heads; p.scale = 0.125f;
-  p.trace = g_trace;
-  set_geometry(p, T, bwd_edge_enabled());
-  const int D = heads * 64;
-  CUtensorMap tq, tqt, td, tdt;
-  int rc = cg_make_tensor_map_bf16(&tq, qkv, (long long)Nimg * T, 3LL * D, 3LL * D, 64);
-  if (rc) return rc;
-  rc = cg_make_tensor_map_bf16(&tqt, qkv, (long long)Nimg * T, 3LL * D, 3LL * D, p.ld_tail);
-  if (rc) return rc;
-  rc = cg_make_tensor_map_bf16(&td, dctx, (long long)Nimg * T, D, D, 64);
-  if (rc) return rc;
-  rc = cg_make_tensor_map_bf16(&tdt, dctx, (long long)Nimg * T, D, D, p.ld_tail);
-  if (rc) return rc;
+// Persistent launch: one CTA per SM walks the Nimg * heads items.  Shared memory: four operand buffers, four staging tiles and
+// `extra` bytes of per-kernel data.  The static cache is per instantiation, i.e. per kernel (function attributes are per kernel and device).
+template <auto kernel, typename... Maps>
+int launch_persistent(AttnParams& p, int Nimg, size_t extra, cudaStream_t s, const Maps&... maps) {
   const size_t opb = (size_t)((p.nblk_ld - 1) * 64 + p.ld_tail) * 128;
-  const size_t smem = 1024 + 4 * opb + 4 * (size_t)TILE_BYTES + BWD_FLOATS * 4 + BBARS_BYTES;
-  p.nitems = Nimg * heads;
-  const int grid = p.nitems < cg_num_sms() ? p.nitems : cg_num_sms();  // persistent: one CTA per SM
-  static size_t configured[CG_MAX_DEVICES] = {};  // function attributes are per device
+  const size_t smem = 1024 + 4 * opb + 4 * (size_t)TILE_BYTES + extra;
+  p.nitems = Nimg * p.heads;
+  const int grid = p.nitems < cg_num_sms() ? p.nitems : cg_num_sms();
+  static size_t configured[CG_MAX_DEVICES] = {};
   const int dev = cg_device_index();
   if (smem > configured[dev]) {
-    CG_CUDA(cudaFuncSetAttribute(attn_bwd_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    CG_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     configured[dev] = smem;
   }
-  CG_CUDA(cg_launch_pdl(attn_bwd_tc_kernel, dim3(grid), dim3(AT_THREADS), smem, s, tq, tqt, td, tdt, p));
+  CG_CUDA(cg_launch_pdl(kernel, dim3(grid), dim3(AT_THREADS), smem, s, maps..., p));
   return 0;
 }
 
 template <bool CAUSAL>
-int launch_attn_fwd_tc(const void* qkv, int Nimg, int T, int heads, void* ctx, float* lse, bool allow_edge, cudaStream_t s) {
+int launch_attn_fwd_tc(const void* qkv, int Nimg, int T, int heads, void* ctx, float* lse, cudaStream_t s) {
   AttnParams p = {};
   p.ctx = reinterpret_cast<__nv_bfloat16*>(ctx);
   p.lse = lse;
-  p.T = T; p.heads = heads; p.scale = 0.125f;
-  p.trace = g_trace;
-  set_geometry(p, T, allow_edge);
-  const int D = heads * 64;
+  set_geometry(p, T, heads, CAUSAL);
   CUtensorMap tq, tqt;
-  int rc = cg_make_tensor_map_bf16(&tq, qkv, (long long)Nimg * T, 3LL * D, 3LL * D, 64);
+  const int rc = make_operand_maps(tq, tqt, qkv, (long long)Nimg * T, 3LL * heads * 64, p);
   if (rc) return rc;
-  rc = cg_make_tensor_map_bf16(&tqt, qkv, (long long)Nimg * T, 3LL * D, 3LL * D, p.ld_tail);
-  if (rc) return rc;
-  const size_t opb = (size_t)((p.nblk_ld - 1) * 64 + p.ld_tail) * 128;
-  const size_t smem = 1024 + 4 * opb + 4 * (size_t)TILE_BYTES + FWD_FLOATS * 4 + FBARS_BYTES;
-  p.nitems = Nimg * heads;
-  const int grid = p.nitems < cg_num_sms() ? p.nitems : cg_num_sms();  // persistent: one CTA per SM
-  static size_t configured[CG_MAX_DEVICES] = {};
-  const int dev = cg_device_index();
-  if (smem > configured[dev]) {  // (one cache per instantiation: function attributes are per kernel)
-    CG_CUDA(cudaFuncSetAttribute(attn_fwd_tc_kernel<CAUSAL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    configured[dev] = smem;
-  }
-  CG_CUDA(cg_launch_pdl(attn_fwd_tc_kernel<CAUSAL>, dim3(grid), dim3(AT_THREADS), smem, s, tq, tqt, p));
-  return 0;
+  return launch_persistent<attn_fwd_tc_kernel<CAUSAL>>(p, Nimg, FWD_FLOATS * 4 + FBARS_BYTES, s, tq, tqt);
 }
 
 }  // namespace
 
-// Return 0 when the tcgen05 path handled the call, 1 when the caller should use the mma.sync kernel (T > 272 or CG_ATTN_TC=0), or an error.
 int cg_attention_fwd_tc(const void* qkv, int Nimg, int T, int heads, void* ctx, float* lse, cudaStream_t s) {
-  if (T > 272 || !tc_enabled()) return 1;
-  return launch_attn_fwd_tc<false>(qkv, Nimg, T, heads, ctx, lse, fwd_edge_enabled(), s);
+  return launch_attn_fwd_tc<false>(qkv, Nimg, T, heads, ctx, lse, s);
 }
 
 // The CLIP text transformer's attention (OpenAI encode_text, utils/functional.py:91-94): tcgen05 path only, no edge token.
 extern "C" int cg_attention_causal_fwd(const void* qkv, int Nseq, int T, int heads, void* ctx, float* lse, void* stream) {
   CG_REQUIRE(qkv && ctx && lse && Nseq > 0 && T > 0 && heads > 0, "cg_attention_causal_fwd: bad arguments");
-  CG_REQUIRE(T <= 272, "cg_attention_causal_fwd: T=%d exceeds the tcgen05 kernel's limit (272)", T);
-  return launch_attn_fwd_tc<true>(qkv, Nseq, T, heads, ctx, lse, false, cg_stream(stream));
+  CG_REQUIRE(T <= ATTN_TC_MAX_T, "cg_attention_causal_fwd: T=%d exceeds the tcgen05 kernel's limit (%d)", T, ATTN_TC_MAX_T);
+  return launch_attn_fwd_tc<true>(qkv, Nseq, T, heads, ctx, lse, cg_stream(stream));
 }
 
 int cg_attention_bwd_tc(const void* qkv, const void* ctx, const void* dctx, const float* lse, int Nimg, int T, int heads, void* dqkv, cudaStream_t s) {
-  if (T > 272 || !tc_enabled()) return 1;
   AttnParams p = {};
   p.lse = const_cast<float*>(lse);
   p.ctx_in = reinterpret_cast<const __nv_bfloat16*>(ctx);
   p.dctx_in = reinterpret_cast<const __nv_bfloat16*>(dctx);
   p.dqkv = reinterpret_cast<__nv_bfloat16*>(dqkv);
-  return launch_attn_bwd_tc(qkv, dctx, Nimg, T, heads, p, s);
+  set_geometry(p, T, heads, false);
+  const int D = heads * 64;
+  CUtensorMap tq, tqt, td, tdt;
+  int rc = make_operand_maps(tq, tqt, qkv, (long long)Nimg * T, 3LL * D, p);
+  if (!rc) rc = make_operand_maps(td, tdt, dctx, (long long)Nimg * T, D, p);
+  if (rc) return rc;
+  return launch_persistent<attn_bwd_tc_kernel>(p, Nimg, BWD_FLOATS * 4 + BBARS_BYTES, s, tq, tqt, td, tdt);
 }
 
 // debug only (tools/trace_attn.py): device buffer of 16 * 64 * 8 int64 that CTA (0,0) of the next launches fills with clock64() stamps

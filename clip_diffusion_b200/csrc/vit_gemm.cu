@@ -533,13 +533,7 @@ int cg_make_tensor_map_bf16(CUtensorMap* out, const void* ptr, long long rows, l
   return 0;
 }
 
-namespace {
-
-int make_tensor_map(CUtensorMap* out, const void* ptr, long long rows, long long cols, long long ld, int box_rows) {
-  return cg_make_tensor_map_bf16(out, ptr, rows, cols, ld, box_rows);
-}
-
-int num_sms() {
+int cg_num_sms() {
   static int per_device[CG_MAX_DEVICES] = {};
   const int dev = cg_device_index();
   if (per_device[dev] == 0) {
@@ -549,6 +543,8 @@ int num_sms() {
   }
   return per_device[dev];
 }
+
+namespace {
 
 template <int BN, int EPI>
 int launch(const CUtensorMap& ta, const CUtensorMap& tb, const GemmArgs& g, cudaStream_t s) {
@@ -560,7 +556,7 @@ int launch(const CUtensorMap& ta, const CUtensorMap& tb, const GemmArgs& g, cuda
     configured[dev] = true;
   }
   const int tiles = ((g.M + BM - 1) / BM) * (g.N / BN);
-  const int grid = tiles < num_sms() ? tiles : num_sms();
+  const int grid = tiles < cg_num_sms() ? tiles : cg_num_sms();
   CG_CUDA(cg_launch_pdl(gemm_bf16_tn_kernel<BN, EPI>, dim3(grid), dim3(NUM_THREADS), smem, s, ta, tb, g));
   return 0;
 }
@@ -590,7 +586,7 @@ int launch_pair(const CUtensorMap& ta, const CUtensorMap& tb, const GemmArgs& g,
     configured[dev] = true;
   }
   const int tiles = ((g.M + 2 * BM - 1) / (2 * BM)) * (g.N / BN2);
-  int clusters = num_sms() / 2;
+  int clusters = cg_num_sms() / 2;
   if (tiles < clusters) clusters = tiles;
   CG_CUDA(cg_launch_pdl(gemm_bf16_tn_pair_kernel<EPI>, dim3(2 * clusters), dim3(NUM_THREADS), smem, s, ta, tb, g));
   return 0;
@@ -632,7 +628,7 @@ int choose_tile(int M, int N, int K, int epilogue) {
   const bool can_pair = can256 && M > 2 * BM;
   if (!can256 || force_bn == 128) return TILE_128;
   if (force_pair == 1 && can_pair) return TILE_PAIR;
-  const int sms = num_sms();
+  const int sms = cg_num_sms();
   const long long mt = (M + BM - 1) / BM, mt2 = (M + 2 * BM - 1) / (2 * BM);
   auto waves = [](long long tiles, long long slots) { return (double)((tiles + slots - 1) / slots); };
   const double c256 = waves(mt * (N / 256), sms) * 256.0;
@@ -676,16 +672,16 @@ extern "C" int cg_gemm_bf16_tn(const void* A, const void* B, int M, int N, int K
                        : 0;
   const int tile = choose_tile(M, N, K, epilogue);
   CUtensorMap ta, tb;
-  int rc = make_tensor_map(&ta, A, M, K, lda, BM);
+  int rc = cg_make_tensor_map_bf16(&ta, A, M, K, lda, BM);
   if (rc) return rc;
   if (tile == TILE_PAIR) {
-    rc = make_tensor_map(&tb, B, N, K, ldb, BN2 / 2);
+    rc = cg_make_tensor_map_bf16(&tb, B, N, K, ldb, BN2 / 2);
     if (rc) return rc;
     GemmArgs gp = {M, N, K, bias, out, aux, (long long)ldo, pos, g2, wide};
     return dispatch_pair(epilogue, ta, tb, gp, cg_stream(stream));
   }
   const int bn = tile == TILE_256 ? 256 : 128;
-  rc = make_tensor_map(&tb, B, N, K, ldb, bn);
+  rc = cg_make_tensor_map_bf16(&tb, B, N, K, ldb, bn);
   if (rc) return rc;
   GemmArgs g = {M, N, K, bias, out, aux, (long long)ldo, pos, g2, wide};
   cudaStream_t s = cg_stream(stream);

@@ -34,7 +34,6 @@ CLIP_CONFIGS = {
     "ViT-L/14": (224, 14, 1024, 24, 16, 768),
     "ViT-L/14@336px": (336, 14, 1024, 24, 16, 768),
 }
-_CLIP_DIMS = {"ViT-B/32": 512, "ViT-B/16": 512, "ViT-L/14": 768, "ViT-L/14@336px": 768}
 
 
 # name: (context_length, vocab_size, width, layers, heads, embed_dim) of the text transformer (OpenAI clip/model.py build_model)
@@ -46,17 +45,31 @@ CLIP_TEXT_CONFIGS = {
 }
 
 
+# leaf names of one residual block's tensors ("<prefix><layer>.<leaf>"), in the order of OpenAI's state dict; the same in both towers
+BLOCK_KEYS = ("attn.in_proj_weight", "attn.in_proj_bias", "attn.out_proj.weight", "attn.out_proj.bias", "mlp.c_fc.weight", "mlp.c_fc.bias",
+              "mlp.c_proj.weight", "mlp.c_proj.bias", "ln_1.weight", "ln_1.bias", "ln_2.weight", "ln_2.bias")
+
+
+def _block_keys(prefix, layers):
+    return ["%s%d.%s" % (prefix, i, k) for i in range(layers) for k in BLOCK_KEYS]
+
+
+def _check_width(width, heads):
+    if width != heads * 64 or width % 128:  # head_dim 64; the GEMMs tile N by 128
+        raise ValueError("width must equal heads*64 and be a multiple of 128")
+
+
 def register_clip_config(name, input_resolution, patch, width, layers, heads, embed_dim):
     """Extra tower shapes (tests use tiny ones).  width must be heads*64 and a multiple of 128."""
-    if width != heads * 64 or width % 128:
-        raise ValueError("width must equal heads*64 and be a multiple of 128")
+    _check_width(width, heads)
     CLIP_CONFIGS[name] = (input_resolution, patch, width, layers, heads, embed_dim)
 
 
 def register_clip_text_config(name, context, vocab, width, layers, heads, embed_dim):
-    """Extra text-tower shapes (tests use tiny ones), same constraints as register_clip_config; context <= 272."""
-    if width != heads * 64 or width % 128 or not 0 < context <= 272:
-        raise ValueError("width must equal heads*64 and be a multiple of 128, and the context length at most 272")
+    """Extra text-tower shapes (tests use tiny ones), same width constraints as register_clip_config; context <= _lib.ATTN_TC_MAX_T."""
+    _check_width(width, heads)
+    if not 0 < context <= _lib.ATTN_TC_MAX_T:
+        raise ValueError("the context length must lie in [1, %d]" % _lib.ATTN_TC_MAX_T)
     CLIP_TEXT_CONFIGS[name] = (context, vocab, width, layers, heads, embed_dim)
 
 
@@ -95,23 +108,19 @@ def random_clip_state_dict(name, seed=1):
 
 def clip_text_state_dict_keys(name):
     """The text-tower keys of an OpenAI CLIP state dict (everything encode_text reads), in OpenAI's naming."""
-    layers = CLIP_TEXT_CONFIGS[name][3]
-    keys = ["token_embedding.weight", "positional_embedding"]
-    for i in range(layers):
-        p = "transformer.resblocks.%d." % i
-        keys += [p + k for k in ("attn.in_proj_weight", "attn.in_proj_bias", "attn.out_proj.weight", "attn.out_proj.bias", "mlp.c_fc.weight",
-                                 "mlp.c_fc.bias", "mlp.c_proj.weight", "mlp.c_proj.bias", "ln_1.weight", "ln_1.bias", "ln_2.weight", "ln_2.bias")]
-    return keys + ["ln_final.weight", "ln_final.bias", "text_projection"]
+    return list(clip_text_state_dict_shapes(name))
 
 
 def clip_text_state_dict_shapes(name):
-    """{key: shape} of the text tower from CLIP_TEXT_CONFIGS, in the order of clip_text_state_dict_keys."""
+    """{key: shape} of the text tower from CLIP_TEXT_CONFIGS, in the order of OpenAI's state dict."""
     context, vocab, width, layers, heads, embed = CLIP_TEXT_CONFIGS[name]
-    known = {"token_embedding.weight": (vocab, width), "positional_embedding": (context, width), "text_projection": (width, embed),
-             "attn.in_proj_weight": (3 * width, width), "attn.in_proj_bias": (3 * width,), "attn.out_proj.weight": (width, width),
+    block = {"attn.in_proj_weight": (3 * width, width), "attn.in_proj_bias": (3 * width,), "attn.out_proj.weight": (width, width),
              "mlp.c_fc.weight": (4 * width, width), "mlp.c_fc.bias": (4 * width,), "mlp.c_proj.weight": (width, 4 * width)}
-    # block keys are looked up by their leaf ("transformer.resblocks.<i>.<leaf>"); every other tensor is [width]
-    return {k: known.get(k.split(".", 3)[-1] if k.startswith("transformer.") else k, (width,)) for k in clip_text_state_dict_keys(name)}
+    shapes = {"token_embedding.weight": (vocab, width), "positional_embedding": (context, width)}
+    # block keys are looked up by their leaf ("transformer.resblocks.<i>.<leaf>"); every other block tensor is [width]
+    shapes.update((k, block.get(k.split(".", 3)[-1], (width,))) for k in _block_keys("transformer.resblocks.", layers))
+    shapes.update({"ln_final.weight": (width,), "ln_final.bias": (width,), "text_projection": (width, embed)})
+    return shapes
 
 
 def random_clip_text_state_dict(name, seed=1):
@@ -151,6 +160,37 @@ def _f32(t, device):
     return t.to(device=device, dtype=torch.float32).contiguous()
 
 
+def _pack_blocks(sd, prefix, layers, device, transposed):
+    """The residual blocks of a state dict under ``prefix``, on the device: each W [N, K] bf16 as the GEMMs' B operand, with
+    ``transposed`` also W^T as the B operand of the dgrad GEMMs; biases and LayerNorm affines fp32."""
+    blocks = []
+    for i in range(layers):
+        p = "%s%d." % (prefix, i)
+        blk = {"ln1": (_f32(sd[p + "ln_1.weight"], device), _f32(sd[p + "ln_1.bias"], device)),
+               "ln2": (_f32(sd[p + "ln_2.weight"], device), _f32(sd[p + "ln_2.bias"], device))}
+        for key, w, b in (("qkv", "attn.in_proj_weight", "attn.in_proj_bias"), ("out", "attn.out_proj.weight", "attn.out_proj.bias"),
+                          ("fc", "mlp.c_fc.weight", "mlp.c_fc.bias"), ("proj", "mlp.c_proj.weight", "mlp.c_proj.bias")):
+            blk["w_" + key], blk["b_" + key] = _bf16(sd[p + w], device), _f32(sd[p + b], device)
+            if transposed:
+                blk["w_" + key + "_t"] = _bf16(sd[p + w].t(), device)
+        blocks.append(blk)
+    return blocks
+
+
+def _block_forward(attention, blk, n, T, heads, x, out, L, h, hg):
+    """One residual block on fp32 [n*T, D] residual streams, x -> out (may be x), with ``attention`` the C-ABI entry point
+    (cg_attention_fwd or cg_attention_causal_fwd).  ``L`` receives the activations the vision backward reads; h, hg are bf16 scratch."""
+    M, D = n * T, x.shape[1]
+    P, C = _lib.ptr, _lib.call
+    C("cg_layernorm_fwd", P(x), P(blk["ln1"][0]), P(blk["ln1"][1]), M, D, D, P(h), None, P(L["mean1"]), P(L["rstd1"]))
+    gemm_bf16_tn(h, blk["w_qkv"], _lib.EPI_BIAS_BF16, bias=blk["b_qkv"], out=L["qkv"])
+    C(attention, P(L["qkv"]), n, T, heads, P(L["ctx"]), P(L["lse"]))
+    gemm_bf16_tn(L["ctx"], blk["w_out"], _lib.EPI_BIAS_RESID_F32, bias=blk["b_out"], out=L["x_mid"], aux=x)
+    C("cg_layernorm_fwd", P(L["x_mid"]), P(blk["ln2"][0]), P(blk["ln2"][1]), M, D, D, P(h), None, P(L["mean2"]), P(L["rstd2"]))
+    gemm_bf16_tn(h, blk["w_fc"], _lib.EPI_BIAS_QGELU_BF16, bias=blk["b_fc"], out=hg, aux=L["u"])
+    gemm_bf16_tn(hg, blk["w_proj"], _lib.EPI_BIAS_RESID_F32, bias=blk["b_proj"], out=out, aux=L["x_mid"])
+
+
 class VisionTransformerB200:
     """Frozen OpenAI-style CLIP vision transformer: forward + input-gradient backward on sm_100a kernels."""
 
@@ -174,28 +214,14 @@ class VisionTransformerB200:
         self.ln_pre = (_f32(sd["visual.ln_pre.weight"], dev), _f32(sd["visual.ln_pre.bias"], dev))
         self.ln_post = (_f32(sd["visual.ln_post.weight"], dev), _f32(sd["visual.ln_post.bias"], dev))
         self.proj = _f32(sd["visual.proj"], dev)
-        self.blocks = []
-        for i in range(layers):
-            p = "visual.transformer.resblocks.%d." % i
-            blk = {
-                "ln1": (_f32(sd[p + "ln_1.weight"], dev), _f32(sd[p + "ln_1.bias"], dev)),
-                "ln2": (_f32(sd[p + "ln_2.weight"], dev), _f32(sd[p + "ln_2.bias"], dev)),
-            }
-            for key, src in (("qkv", "attn.in_proj_weight"), ("out", "attn.out_proj.weight"), ("fc", "mlp.c_fc.weight"), ("proj", "mlp.c_proj.weight")):
-                blk["w_" + key] = _bf16(sd[p + src], dev)
-                blk["w_" + key + "_t"] = _bf16(sd[p + src].t(), dev)
-            blk["b_qkv"] = _f32(sd[p + "attn.in_proj_bias"], dev)
-            blk["b_out"] = _f32(sd[p + "attn.out_proj.bias"], dev)
-            blk["b_fc"] = _f32(sd[p + "mlp.c_fc.bias"], dev)
-            blk["b_proj"] = _f32(sd[p + "mlp.c_proj.bias"], dev)
-            self.blocks.append(blk)
+        self.blocks = _pack_blocks(sd, "visual.transformer.resblocks.", layers, dev, transposed=True)
         self._ws = {}  # persistent activation workspaces per batch size (stable addresses => TMA descriptor cache hits)
         self._generation = 0  # bumped by every forward: the saved activations live in the shared workspace, not in an autograd ctx
         # CUDA graphs: a tower pass is ~7 C-ABI calls per layer and direction on fixed buffers; issuing them one by one costs the host
         # ~12 ms per step for ViT-L/14 (measured: bench.py `host_enqueue_ms_per_step`), which bounds the small configurations and the
         # end-to-end step.  The first pass of a batch size runs eagerly (function attributes, descriptor cache, scratch allocation), the
-        # second is captured, later ones are replayed.  CG_VIT_GRAPHS=0 (or use_graphs = False) keeps every pass eager.
-        self.use_graphs = os.environ.get("CG_VIT_GRAPHS", "1") != "0"
+        # second is captured, later ones are replayed.  use_graphs = False keeps every pass eager.
+        self.use_graphs = True
 
     # ------------------------------------------------------------------ workspaces
     def _workspace(self, n):
@@ -289,13 +315,7 @@ class VisionTransformerB200:
         C("cg_layernorm_fwd", P(ws["x0"]), P(self.ln_pre[0]), P(self.ln_pre[1]), M, D, D, None, P(x), P(ws["mean0"]), P(ws["rstd0"]))
         for i, (blk, L) in enumerate(zip(self.blocks, ws["layers"])):
             x_next = ws["layers"][i + 1]["x_in"] if i + 1 < self.layers else ws["x_out"]
-            C("cg_layernorm_fwd", P(L["x_in"]), P(blk["ln1"][0]), P(blk["ln1"][1]), M, D, D, P(ws["h"]), None, P(L["mean1"]), P(L["rstd1"]))
-            gemm_bf16_tn(ws["h"], blk["w_qkv"], _lib.EPI_BIAS_BF16, bias=blk["b_qkv"], out=L["qkv"])
-            C("cg_attention_fwd", P(L["qkv"]), n, T, self.heads, P(L["ctx"]), P(L["lse"]))
-            gemm_bf16_tn(L["ctx"], blk["w_out"], _lib.EPI_BIAS_RESID_F32, bias=blk["b_out"], out=L["x_mid"], aux=L["x_in"])
-            C("cg_layernorm_fwd", P(L["x_mid"]), P(blk["ln2"][0]), P(blk["ln2"][1]), M, D, D, P(ws["h"]), None, P(L["mean2"]), P(L["rstd2"]))
-            gemm_bf16_tn(ws["h"], blk["w_fc"], _lib.EPI_BIAS_QGELU_BF16, bias=blk["b_fc"], out=ws["hg"], aux=L["u"])
-            gemm_bf16_tn(ws["hg"], blk["w_proj"], _lib.EPI_BIAS_RESID_F32, bias=blk["b_proj"], out=x_next, aux=L["x_mid"])
+            _block_forward("cg_attention_fwd", blk, n, T, self.heads, L["x_in"], x_next, L, ws["h"], ws["hg"])
         # ln_post on the class-token rows (row stride T*D), then the projection
         C("cg_layernorm_fwd", P(ws["x_out"]), P(self.ln_post[0]), P(self.ln_post[1]), n, D, T * D, None, P(ws["y"]), P(ws["meanp"]), P(ws["rstdp"]))
         C("cg_vit_proj_fwd", P(ws["y"]), P(self.proj), n, D, E, P(ws["emb"]))
@@ -368,21 +388,7 @@ class TextTransformerB200:
         self.pos = _f32(sd["positional_embedding"], dev)
         self.ln_final = (_f32(sd["ln_final.weight"], dev), _f32(sd["ln_final.bias"], dev))
         self.proj = _f32(sd["text_projection"], dev)
-        self.blocks = []
-        for i in range(layers):
-            p = "transformer.resblocks.%d." % i
-            blk = {
-                "ln1": (_f32(sd[p + "ln_1.weight"], dev), _f32(sd[p + "ln_1.bias"], dev)),
-                "ln2": (_f32(sd[p + "ln_2.weight"], dev), _f32(sd[p + "ln_2.bias"], dev)),
-            }
-            # W [N, K] bf16 as the GEMM's B operand; no transposed copies (no dgrad)
-            for key, src in (("qkv", "attn.in_proj_weight"), ("out", "attn.out_proj.weight"), ("fc", "mlp.c_fc.weight"), ("proj", "mlp.c_proj.weight")):
-                blk["w_" + key] = _bf16(sd[p + src], dev)
-            blk["b_qkv"] = _f32(sd[p + "attn.in_proj_bias"], dev)
-            blk["b_out"] = _f32(sd[p + "attn.out_proj.bias"], dev)
-            blk["b_fc"] = _f32(sd[p + "mlp.c_fc.bias"], dev)
-            blk["b_proj"] = _f32(sd[p + "mlp.c_proj.bias"], dev)
-            self.blocks.append(blk)
+        self.blocks = _pack_blocks(sd, "transformer.resblocks.", layers, dev, transposed=False)  # no dgrad
 
     def forward_tokens(self, tokens):
         """tokens: int32 [N, context] on the tower's device, ids in [0, vocab) -> embeddings [N, E] fp32."""
@@ -395,26 +401,26 @@ class TextTransformerB200:
         h, qkv, ctx, hg, u, lse = b16(M, D), b16(M, 3 * D), b16(M, D), b16(M, 4 * D), b16(M, 4 * D), f32(n, self.heads, T)
         y, emb = f32(n, D), f32(n, E)
         P, C = _lib.ptr, _lib.call
+        # one set of buffers for every layer, which updates x in place (u: the pre-activation, unused)
+        L = {"mean1": mean, "rstd1": rstd, "qkv": qkv, "ctx": ctx, "lse": lse, "x_mid": x_mid, "mean2": mean, "rstd2": rstd, "u": u}
         C("cg_text_embed_fwd", P(tokens), P(self.token_embedding), P(self.pos), n, T, D, self.vocab_size, P(x))
         for blk in self.blocks:
-            C("cg_layernorm_fwd", P(x), P(blk["ln1"][0]), P(blk["ln1"][1]), M, D, D, P(h), None, P(mean), P(rstd))
-            gemm_bf16_tn(h, blk["w_qkv"], _lib.EPI_BIAS_BF16, bias=blk["b_qkv"], out=qkv)
-            C("cg_attention_causal_fwd", P(qkv), n, T, self.heads, P(ctx), P(lse))
-            gemm_bf16_tn(ctx, blk["w_out"], _lib.EPI_BIAS_RESID_F32, bias=blk["b_out"], out=x_mid, aux=x)
-            C("cg_layernorm_fwd", P(x_mid), P(blk["ln2"][0]), P(blk["ln2"][1]), M, D, D, P(h), None, P(mean), P(rstd))
-            gemm_bf16_tn(h, blk["w_fc"], _lib.EPI_BIAS_QGELU_BF16, bias=blk["b_fc"], out=hg, aux=u)  # (u: the pre-activation, unused)
-            gemm_bf16_tn(hg, blk["w_proj"], _lib.EPI_BIAS_RESID_F32, bias=blk["b_proj"], out=x, aux=x_mid)
+            _block_forward("cg_attention_causal_fwd", blk, n, T, self.heads, x, x, L, h, hg)
         C("cg_text_pool_fwd", P(x), P(tokens), n, T, D, P(self.ln_final[0]), P(self.ln_final[1]), P(y))
         C("cg_vit_proj_fwd", P(y), P(self.proj), n, D, E, P(emb))
         return emb
 
 
+def _require_keys(sd, keys, where, tower):
+    missing = [k for k in keys if k not in sd]
+    if missing:
+        raise KeyError("%s lacks %d %s keys (first: %s): expected OpenAI CLIP naming" % (where, len(missing), tower, missing[0]))
+
+
 def _check_text_state_dict(name, sd, where):
     """KeyError naming the first missing text-tower key, ValueError on a shape that does not match CLIP_TEXT_CONFIGS (host only)."""
     shapes = clip_text_state_dict_shapes(name)
-    missing = [k for k in shapes if k not in sd]
-    if missing:
-        raise KeyError("%s lacks %d text-tower keys (first: %s): expected OpenAI CLIP naming" % (where, len(missing), missing[0]))
+    _require_keys(sd, shapes, where, "text-tower")
     for k, shape in shapes.items():
         if tuple(sd[k].shape) != shape:
             raise ValueError("%s: %s has shape %s, the %s text tower needs %s" % (where, k, tuple(sd[k].shape), name, shape))
@@ -535,9 +541,7 @@ def load_clip_models(model_names, device=None, allow_random_init=False):
         path = os.path.join(wdir, name.replace("/", "_") + ".pt") if wdir else None
         if path and os.path.exists(path):
             sd = torch.load(path, map_location="cpu")
-            missing = [k for k in random_clip_state_dict_keys(name) if k not in sd]
-            if missing:
-                raise KeyError("%s lacks %d visual-tower keys (first: %s): expected OpenAI CLIP naming" % (path, len(missing), missing[0]))
+            _require_keys(sd, random_clip_state_dict_keys(name), path, "visual-tower")
         elif not allow_random_init:
             raise FileNotFoundError(
                 "no weights for %r: set CLIPGUIDE_B200_WEIGHTS to a directory holding %s.pt (OpenAI CLIP state dict), or pass "
@@ -549,13 +553,8 @@ def load_clip_models(model_names, device=None, allow_random_init=False):
 def random_clip_state_dict_keys(name):
     """The ``visual.*`` keys the tower reads from a state dict."""
     _, _, _, layers, _, _ = CLIP_CONFIGS[name]
-    keys = ["visual.conv1.weight", "visual.class_embedding", "visual.positional_embedding", "visual.proj", "visual.ln_pre.weight",
-            "visual.ln_pre.bias", "visual.ln_post.weight", "visual.ln_post.bias"]
-    for i in range(layers):
-        p = "visual.transformer.resblocks.%d." % i
-        keys += [p + k for k in ("attn.in_proj_weight", "attn.in_proj_bias", "attn.out_proj.weight", "attn.out_proj.bias", "mlp.c_fc.weight",
-                                 "mlp.c_fc.bias", "mlp.c_proj.weight", "mlp.c_proj.bias", "ln_1.weight", "ln_1.bias", "ln_2.weight", "ln_2.bias")]
-    return keys
+    return ["visual.conv1.weight", "visual.class_embedding", "visual.positional_embedding", "visual.proj", "visual.ln_pre.weight",
+            "visual.ln_pre.bias", "visual.ln_post.weight", "visual.ln_post.bias"] + _block_keys("visual.transformer.resblocks.", layers)
 
 
 class LinearAestheticPredictor(nn.Module):
@@ -591,7 +590,7 @@ def load_aesthetic_predictors(predictor_names, device=None):
     """models.py:220-240 with seeded random init instead of the downloaded checkpoints."""
     predictors = {}
     for i, name in enumerate(predictor_names):
-        dim = _CLIP_DIMS[name]
+        dim = CLIP_CONFIGS[name][5]
         with torch.random.fork_rng(devices=[]):  # do not disturb the job's global seed (functional.py:105-111)
             torch.manual_seed(100 + i)
             model = MLPAestheticPredictor(dim) if dim == 768 else LinearAestheticPredictor(dim)

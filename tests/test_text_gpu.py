@@ -10,29 +10,37 @@ COS_MIN = 0.999
 NAMES = ["ViT-B/32", "ViT-B/16", "ViT-L/14", "ViT-L/14@336px"]
 
 
-@pytest.mark.parametrize("n,T,heads", [(1, 77, 8), (4, 77, 12), (200, 77, 8),  # (200 x 8 items: more than SMs, several per CTA)
-                                       (2, 1, 2), (2, 2, 2), (2, 63, 2), (2, 64, 2), (2, 65, 2), (1, 128, 2), (2, 129, 2), (1, 200, 3),
-                                       (1, 257, 2), (1, 272, 2)])
-def test_causal_attention_fwd(n, T, heads):
-    from clip_diffusion_b200 import _lib
+CAUSAL_SHAPES = [(1, 77, 8), (4, 77, 12), (200, 77, 8),  # (200 x 8 items: more than SMs, several per CTA)
+                 (2, 1, 2), (2, 2, 2), (2, 63, 2), (2, 64, 2), (2, 65, 2), (1, 128, 2), (2, 129, 2), (1, 200, 3), (1, 257, 2), (1, 272, 2)]
 
-    D = heads * 64
-    g = torch.Generator().manual_seed(T + heads + n)
-    qkv = (torch.randn(n * T, 3 * D, generator=g) * 0.8).bfloat16()
-    q, k, v = [t.float().view(n, T, heads, 64).transpose(1, 2) for t in qkv.split(D, dim=1)]
-    s = (q @ k.transpose(-1, -2)) * 0.125
-    s = s.masked_fill(torch.ones(T, T, dtype=torch.bool).triu(1), float("-inf"))
-    ref = torch.softmax(s, -1) @ v
-    lse_ref = torch.logsumexp(s, -1)
-    P = _lib.ptr
-    qc = qkv.cuda()
-    ctx = torch.full((n * T, D), float("nan"), device="cuda", dtype=torch.bfloat16)
-    lse = torch.full((n, heads, T), float("nan"), device="cuda")
-    _lib.call("cg_attention_causal_fwd", P(qc), n, T, heads, P(ctx), P(lse))
-    out = ctx.float().cpu().view(n, T, heads, 64).transpose(1, 2)
-    assert torch.isfinite(out).all() and torch.isfinite(lse.cpu()).all()
-    assert (out - ref).abs().max().item() < 2e-2 * max(1.0, ref.abs().max().item())
-    assert (lse.cpu() - lse_ref).abs().max().item() < 2e-3
+
+def _causal_cases():
+    """The original shapes on flat inputs; sharp regimes of oracle/attention.py at T = 77 (one block per warpgroup and tile: no rescale
+    possible, a control), 200, 257 and 272, with 1, 4 and 16 heads."""
+    cases = [pytest.param(n, T, heads, "flat", id="%d-%d-%d" % (n, T, heads)) for n, T, heads in CAUSAL_SHAPES]
+    i = 0
+    for regime in ("sharp", "sharp_kmean", "staircase_up", "staircase_down", "huge_pos", "huge_neg", "neighbour", "sink"):
+        for T in (77, 200, 257, 272):
+            heads, n = (1, 4, 16)[i % 3], 3 if regime == "neighbour" else 2
+            i += 1
+            cases.append(pytest.param(n, T, heads, regime, id="%d-%d-%d-%s" % (n, T, heads, regime)))
+    return cases
+
+
+@pytest.mark.parametrize("n,T,heads,regime", _causal_cases())
+def test_causal_attention_fwd(n, T, heads, regime, record_property):
+    """The causal tcgen05 forward against the float64 masked softmax within the error model of oracle/attention.py, in guarded buffers
+    (oracle/attention.py: attention_fwd_guarded).  A sink sits at key 0, which every row keeps."""
+    from oracle import attention as A
+
+    seed = T + heads + n if regime == "flat" else 1000 * n + T + heads
+    qkv, _ = A.make_inputs(regime, n, T, heads, seed, causal=True, **({"pos": 0} if regime == "sink" else {}))
+    qkv = qkv.cuda()
+    ref = A.attention_fwd(*A.split_qkv(qkv, n, T, heads), causal=True)
+    ctx, lse = A.attention_fwd_guarded(qkv, n, T, heads, causal=True)
+    worst = A.worst_ratios({"o": A.rows_to_heads(ctx, n, T, heads), "lse": lse}, ref, A.fwd_bounds(ref))
+    record_property("err_over_bound", {"kernel": "tcgen05 causal", "regime": regime, **worst})
+    assert max(worst.values()) <= 1.0, worst
 
 
 def _prompts(seed, n_extra=3):

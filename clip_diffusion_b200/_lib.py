@@ -23,6 +23,10 @@ EPI_F32 = 4
 EPI_BF16 = 5
 EPI_PATCH_POS_F32 = 6
 
+GEMM_TILE_128x256 = 0
+GEMM_TILE_128x128 = 1
+GEMM_TILE_PAIR_256x256 = 2
+
 
 class CgCut(C.Structure):
     _fields_ = [("y0", C.c_int32), ("x0", C.c_int32), ("size", C.c_int32), ("flags", C.c_int32)]
@@ -79,6 +83,7 @@ _SIGNATURES = {
     "cg_layernorm_fwd": (_I, [_P, _P, _P, _I, _I, _L, _P, _P, _P, _P, _P]),
     "cg_layernorm_bwd": (_I, [_P, _P, _P, _P, _P, _I, _I, _L, _I, _P, _P, _P]),
     "cg_gemm_bf16_tn": (_I, [_P, _P, _I, _I, _I, _L, _L, _I, _P, _P, _P, _L, _P, _I, _P]),
+    "cg_gemm_tile_variant": (_I, [_I, _I, _I, _I]),
     "cg_attention_fwd": (_I, [_P, _I, _I, _I, _P, _P, _P]),
     "cg_attention_bwd": (_I, [_P, _P, _P, _P, _I, _I, _I, _P, _P, _P]),
     "cg_attention_causal_fwd": (_I, [_P, _I, _I, _I, _P, _P, _P]),

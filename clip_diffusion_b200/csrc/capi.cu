@@ -14,7 +14,7 @@ void cg_set_error(const char* fmt, ...) {
 }
 
 extern "C" const char* cg_last_error(void) { return g_err; }
-extern "C" int cg_abi_version(void) { return 4; }  // 4: cg_image_losses_fwd_bwd, deterministic loss values; 3: producer-side GroupNorm partials (input_partial); 2: + UNet NHWC ops (cg_groupnorm_nhwc_*, cg_bias_residual_add_nhwc, cg_resample2x_nhwc, cg_concat2_nhwc)
+extern "C" int cg_abi_version(void) { return 5; }  // 5: cg_gemm_tile_variant; 4: cg_image_losses_fwd_bwd, deterministic loss values; 3: producer-side GroupNorm partials (input_partial); 2: + UNet NHWC ops (cg_groupnorm_nhwc_*, cg_bias_residual_add_nhwc, cg_resample2x_nhwc, cg_concat2_nhwc)
 
 extern "C" int cg_check_device(void) {
   int dev = 0;

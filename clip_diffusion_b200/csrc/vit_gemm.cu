@@ -621,7 +621,7 @@ int env_choice(const char* name) {
   const char* e = getenv(name);
   return e ? atoi(e) : -1;
 }
-enum { TILE_256 = 0, TILE_128 = 1, TILE_PAIR = 2 };
+enum { TILE_256 = CG_GEMM_TILE_128x256, TILE_128 = CG_GEMM_TILE_128x128, TILE_PAIR = CG_GEMM_TILE_PAIR_256x256 };
 int choose_tile(int M, int N, int K, int epilogue) {
   static const int force_pair = env_choice("CG_GEMM_PAIR"), force_bn = env_choice("CG_GEMM_BN");
   const bool can256 = N % 256 == 0;
@@ -643,6 +643,11 @@ int choose_tile(int M, int N, int K, int epilogue) {
 
 }  // namespace
 
+extern "C" int cg_gemm_tile_variant(int M, int N, int K, int epilogue) {
+  CG_REQUIRE(M > 0 && N > 0 && K > 0 && N % 128 == 0, "cg_gemm_tile_variant: bad sizes M=%d N=%d K=%d", M, N, K);
+  return choose_tile(M, N, K, epilogue);
+}
+
 extern "C" int cg_gemm_bf16_tn(const void* A, const void* B, int M, int N, int K, int64_t lda, int64_t ldb, int epilogue, const float* bias,
                                void* out, void* aux, int64_t ldo, const float* pos, int g2, void* stream) {
   CG_REQUIRE(A && B && out, "cg_gemm_bf16_tn: null operand");
@@ -651,6 +656,9 @@ extern "C" int cg_gemm_bf16_tn(const void* A, const void* B, int M, int N, int K
   CG_REQUIRE(N % 128 == 0, "cg_gemm_bf16_tn: N=%d must be a multiple of 128", N);
   CG_REQUIRE(lda % 8 == 0 && ldb % 8 == 0 && lda >= K && ldb >= K, "cg_gemm_bf16_tn: leading dimensions must be >= K and multiples of 8");
   CG_REQUIRE(((uintptr_t)A & 15) == 0 && ((uintptr_t)B & 15) == 0 && ((uintptr_t)out & 15) == 0, "cg_gemm_bf16_tn: pointers must be 16-byte aligned");
+  // the epilogue reads bias, aux and pos with 128-bit (or 256-bit) vector loads
+  CG_REQUIRE(((uintptr_t)bias & 15) == 0 && ((uintptr_t)aux & 15) == 0 && ((uintptr_t)pos & 15) == 0,
+             "cg_gemm_bf16_tn: bias, aux and pos must be 16-byte aligned");
   CG_REQUIRE(ldo % 8 == 0 && ldo >= N, "cg_gemm_bf16_tn: ldo=%lld must be >= N and a multiple of 8", (long long)ldo);
   const bool needs_bias = epilogue == CG_EPI_BIAS_BF16 || epilogue == CG_EPI_BIAS_RESID_F32 || epilogue == CG_EPI_BIAS_QGELU_BF16;
   CG_REQUIRE(!needs_bias || bias, "cg_gemm_bf16_tn: epilogue %d needs a bias", epilogue);

@@ -185,6 +185,7 @@ __global__ void __launch_bounds__(256) patchify_kernel(float* __restrict__ img, 
 }
 
 int rows_grid(int M) { return (M + 7) / 8; }  // 8 warps (rows) per 256-thread block
+bool cg_aligned(const void* p, uintptr_t bytes) { return ((uintptr_t)p & (bytes - 1)) == 0; }  // NULL counts as aligned
 
 }  // namespace
 
@@ -193,6 +194,9 @@ extern "C" int cg_layernorm_fwd(const float* x, const float* gamma, const float*
   CG_REQUIRE(x && gamma && beta && mean && rstd && (y_bf16 || y_f32), "cg_layernorm_fwd: null pointer");
   CG_REQUIRE(M > 0 && D > 0 && D % 128 == 0 && D / 32 <= LN_MAX_PER_LANE, "cg_layernorm_fwd: D=%d must be a multiple of 128 and <= %d", D, 32 * LN_MAX_PER_LANE);
   CG_REQUIRE(row_stride >= D && row_stride % 4 == 0, "cg_layernorm_fwd: bad row stride");
+  // float4 loads of x, gamma, beta and float4 / 4 x bf16 stores of y
+  CG_REQUIRE(cg_aligned(x, 16) && cg_aligned(gamma, 16) && cg_aligned(beta, 16) && cg_aligned(y_f32, 16) && cg_aligned(y_bf16, 8),
+             "cg_layernorm_fwd: x, gamma, beta and y_f32 must be 16-byte aligned, y_bf16 8-byte aligned");
 #define CG_LN_FWD(NV) \
   case NV: CG_CUDA(cg_launch_pdl(ln_fwd_kernel<NV>, dim3(rows_grid(M)), dim3(256), 0, cg_stream(stream), x, gamma, beta, M, D, (long long)row_stride, reinterpret_cast<__nv_bfloat16*>(y_bf16), y_f32, mean, rstd)); break;
   switch (D / 128) {
@@ -209,6 +213,8 @@ extern "C" int cg_layernorm_bwd(const float* dy, const float* x, const float* ga
   CG_REQUIRE(dy && x && gamma && mean && rstd && dx, "cg_layernorm_bwd: null pointer");
   CG_REQUIRE(M > 0 && D > 0 && D % 128 == 0 && D / 32 <= LN_MAX_PER_LANE, "cg_layernorm_bwd: D=%d must be a multiple of 128 and <= %d", D, 32 * LN_MAX_PER_LANE);
   CG_REQUIRE(row_stride >= D && row_stride % 4 == 0, "cg_layernorm_bwd: bad row stride");
+  CG_REQUIRE(cg_aligned(dy, 16) && cg_aligned(x, 16) && cg_aligned(gamma, 16) && cg_aligned(dx, 16) && cg_aligned(dx_bf16, 8),
+             "cg_layernorm_bwd: dy, x, gamma and dx must be 16-byte aligned, dx_bf16 8-byte aligned");
 #define CG_LN_BWD(NV) \
   case NV: CG_CUDA(cg_launch_pdl(ln_bwd_kernel<NV>, dim3(rows_grid(M)), dim3(256), 0, cg_stream(stream), dy, x, gamma, mean, rstd, M, D, (long long)row_stride, accumulate, dx, reinterpret_cast<__nv_bfloat16*>(dx_bf16))); break;
   switch (D / 128) {

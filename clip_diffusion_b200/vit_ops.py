@@ -4,24 +4,49 @@ import torch
 
 from clip_diffusion_b200 import _lib
 
+_F32_OUT = (_lib.EPI_BIAS_RESID_F32, _lib.EPI_F32, _lib.EPI_PATCH_POS_F32)
+_AUX_DTYPE = {_lib.EPI_BIAS_RESID_F32: torch.float32, _lib.EPI_BIAS_QGELU_BF16: torch.bfloat16, _lib.EPI_DQGELU_BF16: torch.bfloat16}
+_NEEDS_BIAS = (_lib.EPI_BIAS_BF16, _lib.EPI_BIAS_RESID_F32, _lib.EPI_BIAS_QGELU_BF16)
+
+
+def _check_matrix(name, t, dtype, rows, cols, device):
+    if t.dtype != dtype or t.dim() != 2 or t.device != device:
+        raise _lib.ClipGuideError("gemm_bf16_tn: %s must be a 2-D %s tensor on %s, got %s %s on %s" % (name, dtype, device, t.dtype, tuple(t.shape), t.device))
+    if t.shape[0] < rows or t.shape[1] < cols or t.stride(1) != 1:
+        raise _lib.ClipGuideError("gemm_bf16_tn: %s must hold at least [%d, %d] with unit column stride, got %s stride %s"
+                                  % (name, rows, cols, tuple(t.shape), t.stride()))
+
 
 def gemm_bf16_tn(a, b, epilogue, bias=None, out=None, aux=None, pos=None, g2=0, m=None):
     """acc[M,N] = a[M,K] @ b[N,K]^T with a fused epilogue (see CG_EPI_* in the header).  a, b: bf16 row-major
-    (row stride may exceed K).  ``out``/``aux`` must be preallocated for in-place / auxiliary epilogues."""
-    _lib.require_cuda(a, b)
+    (row stride may exceed K).  ``out``/``aux`` must be preallocated for in-place / auxiliary epilogues; the kernel
+    addresses ``aux`` with ``out``'s row stride, so both must have the same one."""
+    _lib.require_cuda(a, b, bias, out, aux, pos)
     assert a.dtype == torch.bfloat16 and b.dtype == torch.bfloat16 and a.stride(-1) == 1 and b.stride(-1) == 1
     M = a.shape[0] if m is None else m
     K = a.shape[1]
     N = b.shape[0]
     assert b.shape[1] == K
+    out_dtype = torch.float32 if epilogue in _F32_OUT else torch.bfloat16
     if out is None:
-        dt = torch.float32 if epilogue in (_lib.EPI_F32,) else torch.bfloat16
         assert epilogue != _lib.EPI_PATCH_POS_F32, "the patch epilogue writes into a preallocated token buffer"
-        if epilogue == _lib.EPI_BIAS_RESID_F32:
-            dt = torch.float32
-        out = torch.empty(M, N, device=a.device, dtype=dt)
+        out = torch.empty(M, N, device=a.device, dtype=out_dtype)
     if epilogue == _lib.EPI_BIAS_QGELU_BF16 and aux is None:
         aux = torch.empty(M, N, device=a.device, dtype=torch.bfloat16)
+    out_rows = M // g2 * (g2 + 1) if epilogue == _lib.EPI_PATCH_POS_F32 and g2 > 0 else M
+    _check_matrix("out", out, out_dtype, out_rows, N, a.device)
+    if epilogue in _AUX_DTYPE:
+        if aux is None:
+            raise _lib.ClipGuideError("gemm_bf16_tn: epilogue %d needs aux" % epilogue)
+        _check_matrix("aux", aux, _AUX_DTYPE[epilogue], M, N, a.device)
+        if aux.stride(0) != out.stride(0):
+            raise _lib.ClipGuideError("gemm_bf16_tn: aux row stride %d != out row stride %d" % (aux.stride(0), out.stride(0)))
+    if epilogue in _NEEDS_BIAS:
+        if bias is None or bias.dtype != torch.float32 or not bias.is_contiguous() or bias.shape != (N,) or bias.device != a.device:
+            raise _lib.ClipGuideError("gemm_bf16_tn: epilogue %d needs a contiguous fp32 bias of length %d on %s" % (epilogue, N, a.device))
+    if epilogue == _lib.EPI_PATCH_POS_F32 and (pos is None or pos.dtype != torch.float32 or not pos.is_contiguous()
+                                               or pos.numel() < (g2 + 1) * N or pos.device != a.device):
+        raise _lib.ClipGuideError("gemm_bf16_tn: the patch epilogue needs a contiguous fp32 pos of [g2 + 1, %d] on %s" % (N, a.device))
     _lib.call(
         "cg_gemm_bf16_tn", _lib.ptr(a), _lib.ptr(b), M, N, K, a.stride(0), b.stride(0), epilogue, _lib.ptr(bias), _lib.ptr(out),
         _lib.ptr(aux), out.stride(0), _lib.ptr(pos), g2,

@@ -173,6 +173,13 @@ int cg_layernorm_bwd(const float* dy, const float* x, const float* gamma, const 
 int cg_gemm_bf16_tn(const void* A, const void* B, int M, int N, int K, int64_t lda, int64_t ldb, int epilogue,
                     const float* bias, void* out, void* aux, int64_t ldo, const float* pos, int g2, void* stream);
 
+/* Tile variant cg_gemm_bf16_tn runs a problem on (host only, no launch): the per-problem choice, including the
+ * CG_GEMM_PAIR / CG_GEMM_BN overrides read from the environment at the first call.  Negative on bad sizes. */
+#define CG_GEMM_TILE_128x256 0
+#define CG_GEMM_TILE_128x128 1
+#define CG_GEMM_TILE_PAIR_256x256 2 /* two CTAs of a cluster share one 256 x 256 tile */
+int cg_gemm_tile_variant(int M, int N, int K, int epilogue);
+
 /* Fused multi-head attention over packed qkv [Nimg*T, 3*D] bf16 (q | k | v, head h at column h*64), head_dim 64,
  * softmax scale 1/8.  ctx [Nimg*T, D] bf16, lse [Nimg, heads, T] fp32. */
 int cg_attention_fwd(const void* qkv, int Nimg, int T, int heads, void* ctx, float* lse, void* stream);

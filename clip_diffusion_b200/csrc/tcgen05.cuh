@@ -82,6 +82,11 @@ __device__ __forceinline__ uint64_t make_smem_desc(uint32_t smem_addr) {
   d |= (uint64_t)2 << 61;
   return d;
 }
+// Instruction descriptor, kind::f16: D fp32 (bit 4), A/B bf16 (bits 7, 10), A K-major, B K-major or MN-major (bit 16),
+// N>>3 at bit 17, M>>4 at bit 24.
+__host__ __device__ constexpr uint32_t idesc_bf16(int m, int n, bool b_mn_major) {
+  return (1u << 4) | (1u << 7) | (1u << 10) | (b_mn_major ? (1u << 16) : 0u) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(m >> 4) << 24);
+}
 
 
 __device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }

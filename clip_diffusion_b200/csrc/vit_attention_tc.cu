@@ -89,10 +89,6 @@ __device__ __forceinline__ uint32_t elect_one() {
   asm volatile("{\n\t.reg .pred P;\n\telect.sync _|P, 0xffffffff;\n\tselp.u32 %0, 1, 0, P;\n\t}" : "=r"(pred));
   return pred;
 }
-// instruction descriptor, kind::f16: D fp32 (bit 4), A/B bf16 (bits 7, 10), b_major (bit 16: MN-major B), N>>3 at 17, M>>4 at 24
-__device__ __forceinline__ uint32_t idesc_bf16(int n, bool b_mn_major) {
-  return (1u << 4) | (1u << 7) | (1u << 10) | (b_mn_major ? (1u << 16) : 0u) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
-}
 __device__ __forceinline__ void st_shared_v4(uint32_t a, uint32_t x, uint32_t y, uint32_t z, uint32_t w) {
   asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(a), "r"(x), "r"(y), "r"(z), "r"(w) : "memory");
 }
@@ -503,7 +499,7 @@ __global__ void __launch_bounds__(AT_THREADS, 1)
   } else if (warp < 2) {
     // ================= S issuers (warp-converged loops, elected lane): warp = parity of the running block index
     const uint32_t elected = elect_one();
-    const uint32_t id_full = idesc_bf16(64, false), id_tail = idesc_bf16(p.tail_rows, false);
+    const uint32_t id_full = idesc_bf16(128, 64, false), id_tail = idesc_bf16(128, p.tail_rows, false);
     int it = 0, gg0 = 0;
     for (int w = blockIdx.x; w < nitems; w += gridDim.x, ++it, gg0 += G) {
       const uint32_t opar = (uint32_t)it & 1u;
@@ -550,7 +546,7 @@ __global__ void __launch_bounds__(AT_THREADS, 1)
   } else if (warp == 2) {
     // ================= P V issuer
     const uint32_t elected = elect_one();
-    const uint32_t id_acc = idesc_bf16(64, true);
+    const uint32_t id_acc = idesc_bf16(128, 64, true);
     uint32_t accpar = 0;  // bit a: parity of the use count of accumulator slot a
     int it = 0, gg0 = 0;
     for (int w = blockIdx.x; w < nitems; w += gridDim.x, ++it, gg0 += G) {
@@ -1001,7 +997,7 @@ __global__ void __launch_bounds__(AT_THREADS, 1)
   if (warp < 4) {
     // ================= four MMA issuer warps (warp-converged loops, elected lane); warp 3 is also the TMA producer
     const uint32_t elected = elect_one();
-    const uint32_t id_full = idesc_bf16(64, false), id_tail = idesc_bf16(p.tail_rows, false), id_acc = idesc_bf16(64, true);
+    const uint32_t id_full = idesc_bf16(128, 64, false), id_tail = idesc_bf16(128, p.tail_rows, false), id_acc = idesc_bf16(128, 64, true);
     uint32_t cuse = 0;  // accumulator issuers: bit a = parity of the number of uses of slot a issued so far
     int it = 0, gg0 = 0;
     for (int w = blockIdx.x; w < nitems; w += gridDim.x, ++it, gg0 += G) {

@@ -1,12 +1,14 @@
 // bf16 GEMM for the CLIP ViT (QKV / out-proj / MLP / patch-embed and their dgrads) on the 5th-gen tensor
 // cores of sm_100a:  acc[M,N] = A[M,K] . B[N,K]^T,  fp32 accumulation in TMEM, fused epilogues.
 //
-//   * operands staged by TMA (cp.async.bulk.tensor, 128B swizzle) into a 4-stage shared-memory ring;
-//   * one elected thread issues tcgen05.mma (cta_group::1, M=128, N=BN, K=16 per instruction);
+//   * three tile variants from one kernel body: 128x256 and 128x128 on one CTA (cta_group::1, M=128), 256x256 on a
+//     CTA pair (cta_group::2, M=256, see gemm_body);
+//   * operands staged by TMA (cp.async.bulk.tensor, 128B swizzle) into a shared-memory ring;
+//   * one elected thread issues tcgen05.mma (N=BN, K=16 per instruction);
 //   * the accumulator lives in TMEM and is double buffered (2 x BN columns), so the epilogue of tile i
 //     overlaps the main loop of tile i+1;
-//   * persistent: one CTA per SM walks the tile list (tile = blockIdx.x + i*gridDim.x), consecutive
-//     tiles share the A row-block so it is reused out of L2;
+//   * persistent: each CTA (or CTA pair) c of n walks the tile list (tile = c + i*n), consecutive tiles share the
+//     A row-block so it is reused out of L2;
 //   * warp roles: 0 = TMA producer, 1 = MMA issuer, 2 = TMEM allocator, 4..11 = epilogue (tcgen05.ld ->
 //     registers -> bias / QuickGELU / residual -> global).  Eight epilogue warps = two per scheduler and per
 //     TMEM lane quarter (each takes half of the tile's columns): one warp per scheduler cannot hide its own ALU
@@ -25,7 +27,6 @@ namespace {
 
 constexpr int BM = 128;
 constexpr int BK = 64;  // 64 bf16 = 128 bytes = one swizzle atom row
-constexpr int STAGES = 4;
 constexpr int NUM_EPI_WARPS = 8;
 constexpr int NUM_THREADS = 128 + 32 * NUM_EPI_WARPS;
 
@@ -41,11 +42,6 @@ struct GemmArgs {
 };
 
 using namespace tc;
-
-// Instruction descriptor for kind::f16: D fp32, A/B bf16, both K-major, M=128, N=BN.
-__host__ __device__ constexpr uint32_t make_idesc(int n) {
-  return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(BM >> 4) << 24);
-}
 
 // sigmoid(1.702 u) = 0.5 * tanh(0.851 u) + 0.5 : one MUFU op instead of ex2 + a full-precision division
 __device__ __forceinline__ float sigmoid_1702(float u) {
@@ -176,137 +172,11 @@ __device__ __forceinline__ void epilogue_chunk(const GemmArgs& g, long long row,
   }
 }
 
-template <int BN, int EPI>
-__global__ void __launch_bounds__(NUM_THREADS, 1) gemm_bf16_tn_kernel(const __grid_constant__ CUtensorMap tmA,
-                                                                       const __grid_constant__ CUtensorMap tmB, const GemmArgs g) {
-  extern __shared__ __align__(1024) uint8_t smem_raw[];
-  constexpr uint32_t A_BYTES = BM * BK * 2;
-  constexpr uint32_t B_BYTES = BN * BK * 2;
-  constexpr uint32_t STAGE_BYTES = A_BYTES + B_BYTES;
-  constexpr uint32_t TMEM_COLS = 2 * BN;  // 256 or 512: power of two >= 32
-
-  // 1024-byte alignment for the 128B swizzle
-  const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-  const uint32_t bar_base = smem_base + STAGES * STAGE_BYTES;
-  // barriers: full[STAGES], empty[STAGES], tmem_full[2], tmem_empty[2]; then the TMEM base address word
-  auto full_bar = [&](int s) { return bar_base + 8u * s; };
-  auto empty_bar = [&](int s) { return bar_base + 8u * (STAGES + s); };
-  auto tfull_bar = [&](int s) { return bar_base + 8u * (2 * STAGES + s); };
-  auto tempty_bar = [&](int s) { return bar_base + 8u * (2 * STAGES + 2 + s); };
-  const uint32_t tmem_slot = bar_base + 8u * (2 * STAGES + 4);
-
-  cg_griddep_launch();
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int m_tiles = (g.M + BM - 1) / BM, n_tiles = g.N / BN;
-  const int num_tiles = m_tiles * n_tiles;
-  const int k_blocks = g.K / BK;
-
-  if (warp == 0 && lane == 0) {
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&tmA) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&tmB) : "memory");
-  }
-  if (warp == 1 && lane == 0) {
-    for (int s = 0; s < STAGES; ++s) { mbar_init(full_bar(s), 1); mbar_init(empty_bar(s), 1); }
-    for (int s = 0; s < 2; ++s) { mbar_init(tfull_bar(s), 1); mbar_init(tempty_bar(s), NUM_EPI_WARPS); }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 2) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tmem_slot), "r"(TMEM_COLS) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  cg_griddep_wait();  // prologue done: from here on the predecessor's output is read (and buffers it may still read are written)
-  tcgen05_fence_before();
-  __syncthreads();
-  tcgen05_fence_after();
-  uint32_t tmem_base;
-  asm volatile("ld.shared.b32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot) : "memory");
-
-  if (warp == 0) {
-    // ================= TMA producer =================
-    if (lane == 0) {
-      int stage = 0;
-      uint32_t phase = 0;
-      for (int t = blockIdx.x; t < num_tiles; t += gridDim.x) {
-        const int m_blk = t / n_tiles, n_blk = t - m_blk * n_tiles;
-        for (int kb = 0; kb < k_blocks; ++kb) {
-          mbar_wait(empty_bar(stage), phase ^ 1u);
-          const uint32_t a_dst = smem_base + stage * STAGE_BYTES, b_dst = a_dst + A_BYTES;
-          mbar_arrive_expect_tx(full_bar(stage), STAGE_BYTES);
-          tma_load_2d(a_dst, &tmA, full_bar(stage), kb * BK, m_blk * BM);
-          tma_load_2d(b_dst, &tmB, full_bar(stage), kb * BK, n_blk * BN);
-          if (++stage == STAGES) { stage = 0; phase ^= 1u; }
-        }
-      }
-    }
-  } else if (warp == 1) {
-    // ================= MMA issuer =================
-    if (lane == 0) {
-      constexpr uint32_t idesc = make_idesc(BN);
-      int stage = 0;
-      uint32_t phase = 0;
-      int it = 0;
-      for (int t = blockIdx.x; t < num_tiles; t += gridDim.x, ++it) {
-        const int as = it & 1;
-        const uint32_t aphase = (uint32_t)(it >> 1) & 1u;
-        mbar_wait(tempty_bar(as), aphase ^ 1u);  // epilogue has drained this accumulator
-        tcgen05_fence_after();
-        const uint32_t d_tmem = tmem_base + (uint32_t)(as * BN);
-        for (int kb = 0; kb < k_blocks; ++kb) {
-          mbar_wait(full_bar(stage), phase);
-          tcgen05_fence_after();
-          const uint32_t a_addr = smem_base + stage * STAGE_BYTES, b_addr = a_addr + A_BYTES;
-          const uint64_t adesc = make_smem_desc(a_addr), bdesc = make_smem_desc(b_addr);
-#pragma unroll
-          for (int k = 0; k < BK / 16; ++k) {
-            // advance 16 elements = 32 bytes along K inside the swizzle atom: +2 in the (addr >> 4) field
-            umma_bf16(d_tmem, adesc + (uint64_t)(2 * k), bdesc + (uint64_t)(2 * k), idesc, (kb | k) != 0 ? 1u : 0u);
-          }
-          umma_commit(empty_bar(stage));  // smem slot free once these MMAs have read it
-          if (kb == k_blocks - 1) umma_commit(tfull_bar(as));
-          if (++stage == STAGES) { stage = 0; phase ^= 1u; }
-        }
-      }
-    }
-  } else if (warp >= 4) {
-    // ================= epilogue =================
-    const int q = warp & 3;             // TMEM lane quarter this warp may touch (warp id % 4)
-    const int chalf = (warp - 4) >> 2;  // which half of the tile's columns this warp drains
-    int it = 0;
-    for (int t = blockIdx.x; t < num_tiles; t += gridDim.x, ++it) {
-      const int m_blk = t / n_tiles, n_blk = t - m_blk * n_tiles;
-      const int as = it & 1;
-      const uint32_t aphase = (uint32_t)(it >> 1) & 1u;
-      mbar_wait(tfull_bar(as), aphase);
-      tcgen05_fence_after();
-      const long long row = (long long)m_blk * BM + q * 32 + lane;
-      long long orow = row;
-      if (EPI == CG_EPI_PATCH_POS_F32) orow = (row / g.g2) * (g.g2 + 1) + 1 + row % g.g2;
-      const uint32_t t_row = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(as * BN);
-#pragma unroll 1
-      for (int c = chalf * (BN / 2); c < (chalf + 1) * (BN / 2); c += 32) {
-        uint32_t acc[32];
-        tmem_ld32(t_row + (uint32_t)c, acc);
-        tmem_ld_wait();
-        if (row < g.M) epilogue_chunk<EPI>(g, row, orow, n_blk * BN + c, acc);
-      }
-      tcgen05_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive(tempty_bar(as));
-    }
-  }
-  tcgen05_fence_before();
-  __syncthreads();
-  if (warp == 2) {
-    tcgen05_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(TMEM_COLS) : "memory");
-  }
-}
-
-// ---------------------------------------------------------------------------------- CTA-pair variant
+// ---------------------------------------------------------------------------------- CTA-pair pieces
 // cta_group::2: two CTAs of one cluster (one TPC) share a 256x256 output tile.  Each CTA stages ITS 128 rows of A and
 // HALF of the B tile (128 of the 256 output columns); the leader CTA issues tcgen05.mma.cta_group::2 (M=256), which
 // reads both halves of B from both SMs' shared memory, so per 64-deep k-block the pair pulls 64 KB from L2 instead of
-// 2 x 48 KB -- the single-CTA kernel is L2->smem bound at ~1.0-1.15 PFLOP/s (profiles/).  6-stage ring (32 KB/stage).
+// 2 x 48 KB -- the single-CTA kernel is L2->smem bound at ~1.0-1.15 PFLOP/s (profiles/).
 __device__ __forceinline__ uint32_t cluster_ctarank() {
   uint32_t r;
   asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
@@ -344,135 +214,189 @@ __device__ __forceinline__ void umma_bf16_pair(uint32_t tmem_d, uint64_t adesc, 
       : "memory");
 }
 
-constexpr int STAGES2 = 6;
-constexpr int BN2 = 256;
+// ---------------------------------------------------------------------------------- kernel
+// A stage holds this CTA's BM rows of A and its BN / CTAS rows of B: 48 KB for 128x256, 32 KB for a pair CTA, so a
+// pair runs a 6-stage ring in the shared memory that holds 4 stages of 128x256.
+template <int CTAS>
+constexpr int STAGES = CTAS == 2 ? 6 : 4;
+template <int BN, int CTAS>
+constexpr uint32_t STAGE_BYTES = (BM + BN / CTAS) * BK * 2;
+template <int BN, int CTAS>
+constexpr size_t SMEM_BYTES = (size_t)STAGES<CTAS> * STAGE_BYTES<BN, CTAS> + 1024 /*align slack*/ + 256 /*barriers*/;
 
-template <int EPI>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1)
-    gemm_bf16_tn_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const GemmArgs g) {
+// One body for every tile variant: BN is the output tile's width; CTAS = 1, or 2 for a CTA pair (a cluster of two)
+// sharing a 2*BM x BN tile.
+template <int BN, int CTAS, int EPI>
+__device__ __forceinline__ void gemm_body(const CUtensorMap& tmA, const CUtensorMap& tmB, const GemmArgs& g) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
-  constexpr uint32_t A_BYTES = BM * BK * 2;         // this CTA's 128 rows of A
-  constexpr uint32_t B_BYTES = (BN2 / 2) * BK * 2;  // this CTA's half of the B tile
-  constexpr uint32_t STAGE_BYTES = A_BYTES + B_BYTES;
-  constexpr uint32_t TMEM_COLS = 2 * BN2;
+  constexpr int ST = STAGES<CTAS>;
+  constexpr uint32_t A_BYTES = BM * BK * 2;
+  constexpr uint32_t STAGE = STAGE_BYTES<BN, CTAS>;
+  constexpr uint32_t TMEM_COLS = 2 * BN;  // 256 or 512: power of two >= 32
 
+  // 1024-byte alignment for the 128B swizzle
   const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-  const uint32_t bar_base = smem_base + STAGES2 * STAGE_BYTES;
+  const uint32_t bar_base = smem_base + ST * STAGE;
+  // barriers: full[ST], empty[ST], tmem_full[2], tmem_empty[2]; then the TMEM base address word
   auto full_bar = [&](int s) { return bar_base + 8u * s; };
-  auto empty_bar = [&](int s) { return bar_base + 8u * (STAGES2 + s); };
-  auto tfull_bar = [&](int s) { return bar_base + 8u * (2 * STAGES2 + s); };
-  auto tempty_bar = [&](int s) { return bar_base + 8u * (2 * STAGES2 + 2 + s); };
-  const uint32_t tmem_slot = bar_base + 8u * (2 * STAGES2 + 4);
+  auto empty_bar = [&](int s) { return bar_base + 8u * (ST + s); };
+  auto tfull_bar = [&](int s) { return bar_base + 8u * (2 * ST + s); };
+  auto tempty_bar = [&](int s) { return bar_base + 8u * (2 * ST + 2 + s); };
+  const uint32_t tmem_slot = bar_base + 8u * (2 * ST + 4);
 
   cg_griddep_launch();
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const uint32_t rank = cluster_ctarank();
+  uint32_t rank = 0;  // CTA of the pair: it stages rows rank*BM.. of the tile's A and columns rank*BN/2.. of its B
+  if constexpr (CTAS == 2) rank = cluster_ctarank();
   const bool leader = rank == 0;
-  const int m_tiles = (g.M + 2 * BM - 1) / (2 * BM), n_tiles = g.N / BN2;
+  const int m_tiles = (g.M + CTAS * BM - 1) / (CTAS * BM), n_tiles = g.N / BN;
   const int num_tiles = m_tiles * n_tiles;
   const int k_blocks = g.K / BK;
+  // The tile walk.  A single CTA reads blockIdx / gridDim inside each role's loop, where the compiler keeps the walk on
+  // the uniform datapath; a pair reads its cluster index once.
   const int cluster_id = blockIdx.x >> 1, num_clusters = gridDim.x >> 1;
+  auto first_tile = [&] { return CTAS == 2 ? cluster_id : (int)blockIdx.x; };
+  auto tile_step = [&] { return CTAS == 2 ? num_clusters : (int)gridDim.x; };
 
   if (warp == 0 && lane == 0) {
     asm volatile("prefetch.tensormap [%0];" ::"l"(&tmA) : "memory");
     asm volatile("prefetch.tensormap [%0];" ::"l"(&tmB) : "memory");
   }
   if (warp == 1 && lane == 0) {
-    for (int s = 0; s < STAGES2; ++s) { mbar_init(full_bar(s), 1); mbar_init(empty_bar(s), 1); }
-    for (int s = 0; s < 2; ++s) { mbar_init(tfull_bar(s), 1); mbar_init(tempty_bar(s), 2 * NUM_EPI_WARPS); }
+    for (int s = 0; s < ST; ++s) { mbar_init(full_bar(s), 1); mbar_init(empty_bar(s), 1); }
+    for (int s = 0; s < 2; ++s) { mbar_init(tfull_bar(s), 1); mbar_init(tempty_bar(s), CTAS * NUM_EPI_WARPS); }
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
   if (warp == 2) {
-    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tmem_slot), "r"(TMEM_COLS) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
+    if constexpr (CTAS == 2) {
+      asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tmem_slot), "r"(TMEM_COLS) : "memory");
+      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
+    } else {
+      asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tmem_slot), "r"(TMEM_COLS) : "memory");
+      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    }
   }
-  cg_griddep_wait();
+  cg_griddep_wait();  // prologue done: from here on the predecessor's output is read (and buffers it may still read are written)
   tcgen05_fence_before();
-  cluster_sync_all();
+  if constexpr (CTAS == 2) cluster_sync_all(); else __syncthreads();
   tcgen05_fence_after();
   uint32_t tmem_base;
   asm volatile("ld.shared.b32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot) : "memory");
 
   if (warp == 0) {
-    // ================= TMA producer (both CTAs): data into OWN smem, bytes reported to the LEADER's full barrier
+    // ================= TMA producer: a pair CTA loads into its own smem and reports the bytes to the LEADER's full barrier
     if (lane == 0) {
       int stage = 0;
       uint32_t phase = 0;
-      for (int t = cluster_id; t < num_tiles; t += num_clusters) {
+      for (int t = first_tile(); t < num_tiles; t += tile_step()) {
         const int m_blk = t / n_tiles, n_blk = t - m_blk * n_tiles;
-        const int m0 = m_blk * 2 * BM + (int)rank * BM;
-        const int n0 = n_blk * BN2 + (int)rank * (BN2 / 2);
+        const int m0 = m_blk * CTAS * BM + (int)rank * BM;
+        const int n0 = n_blk * BN + (int)rank * (BN / CTAS);
         for (int kb = 0; kb < k_blocks; ++kb) {
           mbar_wait(empty_bar(stage), phase ^ 1u);
-          const uint32_t a_dst = smem_base + stage * STAGE_BYTES, b_dst = a_dst + A_BYTES;
-          if (leader) mbar_arrive_expect_tx(full_bar(stage), 2 * STAGE_BYTES);
-          const uint32_t lead_bar = map_to_cta(full_bar(stage), 0);
-          tma_load_2d_pair(a_dst, &tmA, lead_bar, kb * BK, m0);
-          tma_load_2d_pair(b_dst, &tmB, lead_bar, kb * BK, n0);
-          if (++stage == STAGES2) { stage = 0; phase ^= 1u; }
+          const uint32_t a_dst = smem_base + stage * STAGE, b_dst = a_dst + A_BYTES;
+          if constexpr (CTAS == 2) {
+            if (leader) mbar_arrive_expect_tx(full_bar(stage), 2 * STAGE);
+            const uint32_t lead_bar = map_to_cta(full_bar(stage), 0);
+            tma_load_2d_pair(a_dst, &tmA, lead_bar, kb * BK, m0);
+            tma_load_2d_pair(b_dst, &tmB, lead_bar, kb * BK, n0);
+          } else {
+            mbar_arrive_expect_tx(full_bar(stage), STAGE);
+            tma_load_2d(a_dst, &tmA, full_bar(stage), kb * BK, m0);
+            tma_load_2d(b_dst, &tmB, full_bar(stage), kb * BK, n0);
+          }
+          if (++stage == ST) { stage = 0; phase ^= 1u; }
         }
       }
     }
   } else if (warp == 1) {
-    // ================= MMA issuer (leader CTA only)
+    // ================= MMA issuer (the leader CTA of a pair)
     if (leader && lane == 0) {
-      constexpr uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(BN2 >> 3) << 17) | ((uint32_t)((2 * BM) >> 4) << 24);
+      constexpr uint32_t idesc = idesc_bf16(CTAS * BM, BN, false);
       int stage = 0;
       uint32_t phase = 0;
       int it = 0;
-      for (int t = cluster_id; t < num_tiles; t += num_clusters, ++it) {
+      for (int t = first_tile(); t < num_tiles; t += tile_step(), ++it) {
         const int as = it & 1;
         const uint32_t aphase = (uint32_t)(it >> 1) & 1u;
-        mbar_wait(tempty_bar(as), aphase ^ 1u);  // both CTAs' epilogues have drained this accumulator
+        mbar_wait(tempty_bar(as), aphase ^ 1u);  // the epilogue (of both CTAs) has drained this accumulator
         tcgen05_fence_after();
-        const uint32_t d_tmem = tmem_base + (uint32_t)(as * BN2);
+        const uint32_t d_tmem = tmem_base + (uint32_t)(as * BN);
         for (int kb = 0; kb < k_blocks; ++kb) {
           mbar_wait(full_bar(stage), phase);
           tcgen05_fence_after();
-          const uint32_t a_addr = smem_base + stage * STAGE_BYTES, b_addr = a_addr + A_BYTES;
+          const uint32_t a_addr = smem_base + stage * STAGE, b_addr = a_addr + A_BYTES;
           const uint64_t adesc = make_smem_desc(a_addr), bdesc = make_smem_desc(b_addr);
 #pragma unroll
-          for (int k = 0; k < BK / 16; ++k)
-            umma_bf16_pair(d_tmem, adesc + (uint64_t)(2 * k), bdesc + (uint64_t)(2 * k), idesc, (kb | k) != 0 ? 1u : 0u);
-          umma_commit_pair(empty_bar(stage));  // frees the slot in BOTH CTAs
-          if (kb == k_blocks - 1) umma_commit_pair(tfull_bar(as));
-          if (++stage == STAGES2) { stage = 0; phase ^= 1u; }
+          for (int k = 0; k < BK / 16; ++k) {
+            // advance 16 elements = 32 bytes along K inside the swizzle atom: +2 in the (addr >> 4) field
+            const uint64_t ad = adesc + (uint64_t)(2 * k), bd = bdesc + (uint64_t)(2 * k);
+            if constexpr (CTAS == 2) umma_bf16_pair(d_tmem, ad, bd, idesc, (kb | k) != 0 ? 1u : 0u);
+            else umma_bf16(d_tmem, ad, bd, idesc, (kb | k) != 0 ? 1u : 0u);
+          }
+          // the smem slot is free once these MMAs have read it; a pair's commit multicasts to both CTAs, whose
+          // producers each wait on their own empty barrier
+          if constexpr (CTAS == 2) {
+            umma_commit_pair(empty_bar(stage));
+            if (kb == k_blocks - 1) umma_commit_pair(tfull_bar(as));
+          } else {
+            umma_commit(empty_bar(stage));
+            if (kb == k_blocks - 1) umma_commit(tfull_bar(as));
+          }
+          if (++stage == ST) { stage = 0; phase ^= 1u; }
         }
       }
     }
   } else if (warp >= 4) {
-    // ================= epilogue (both CTAs, own 128 rows)
-    const int q = warp & 3;
-    const int chalf = (warp - 4) >> 2;
+    // ================= epilogue (a pair CTA drains its own 128 rows)
+    const int q = warp & 3;             // TMEM lane quarter this warp may touch (warp id % 4)
+    const int chalf = (warp - 4) >> 2;  // which half of the tile's columns this warp drains
     int it = 0;
-    for (int t = cluster_id; t < num_tiles; t += num_clusters, ++it) {
+    for (int t = first_tile(); t < num_tiles; t += tile_step(), ++it) {
       const int m_blk = t / n_tiles, n_blk = t - m_blk * n_tiles;
       const int as = it & 1;
       const uint32_t aphase = (uint32_t)(it >> 1) & 1u;
       mbar_wait(tfull_bar(as), aphase);
       tcgen05_fence_after();
-      const long long row = (long long)m_blk * 2 * BM + (long long)rank * BM + q * 32 + lane;
+      const long long row = (long long)m_blk * CTAS * BM + (long long)rank * BM + q * 32 + lane;
       long long orow = row;
       if (EPI == CG_EPI_PATCH_POS_F32) orow = (row / g.g2) * (g.g2 + 1) + 1 + row % g.g2;
-      const uint32_t t_row = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(as * BN2);
+      const uint32_t t_row = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(as * BN);
 #pragma unroll 1
-      for (int c = chalf * (BN2 / 2); c < (chalf + 1) * (BN2 / 2); c += 32) {
+      for (int c = chalf * (BN / 2); c < (chalf + 1) * (BN / 2); c += 32) {
         uint32_t acc[32];
         tmem_ld32(t_row + (uint32_t)c, acc);
         tmem_ld_wait();
-        if (row < g.M) epilogue_chunk<EPI>(g, row, orow, n_blk * BN2 + c, acc);
+        if (row < g.M) epilogue_chunk<EPI>(g, row, orow, n_blk * BN + c, acc);
       }
       tcgen05_fence_before();
       __syncwarp();
-      if (lane == 0) mbar_arrive_remote(map_to_cta(tempty_bar(as), 0));
+      if (lane == 0) {
+        if constexpr (CTAS == 2) mbar_arrive_remote(map_to_cta(tempty_bar(as), 0));
+        else mbar_arrive(tempty_bar(as));
+      }
     }
   }
   tcgen05_fence_before();
-  cluster_sync_all();  // nobody leaves (or frees TMEM) while the peer may still read this CTA's shared memory
+  if constexpr (CTAS == 2) cluster_sync_all();  // nobody leaves (or frees TMEM) while the peer may still read this CTA's shared memory
+  else __syncthreads();
   if (warp == 2) {
     tcgen05_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(TMEM_COLS) : "memory");
+    if constexpr (CTAS == 2) asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(TMEM_COLS) : "memory");
+    else asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(TMEM_COLS) : "memory");
   }
+}
+
+// Two entries, so that only the pair kernels carry the cluster shape (single-CTA kernels do not launch as clusters of one)
+template <int BN, int EPI>
+__global__ void __launch_bounds__(NUM_THREADS, 1) gemm_bf16_tn_kernel(const __grid_constant__ CUtensorMap tmA,
+                                                                       const __grid_constant__ CUtensorMap tmB, const GemmArgs g) {
+  gemm_body<BN, 1, EPI>(tmA, tmB, g);
+}
+template <int EPI>
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1)
+    gemm_bf16_tn_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const GemmArgs g) {
+  gemm_body<256, 2, EPI>(tmA, tmB, g);
 }
 
 // ---------------------------------------------------------------------------------- host side
@@ -546,61 +470,33 @@ int cg_num_sms() {
 
 namespace {
 
-template <int BN, int EPI>
+template <int BN, int CTAS, int EPI>
 int launch(const CUtensorMap& ta, const CUtensorMap& tb, const GemmArgs& g, cudaStream_t s) {
-  constexpr size_t smem = (size_t)STAGES * (BM * BK * 2 + BN * BK * 2) + 1024 /*align slack*/ + 256 /*barriers*/;
+  constexpr auto kernel = CTAS == 2 ? gemm_bf16_tn_pair_kernel<EPI> : gemm_bf16_tn_kernel<BN, EPI>;
+  constexpr size_t smem = SMEM_BYTES<BN, CTAS>;
   static bool configured[CG_MAX_DEVICES] = {};  // function attributes are per device
   const int dev = cg_device_index();
   if (!configured[dev]) {
-    CG_CUDA(cudaFuncSetAttribute(gemm_bf16_tn_kernel<BN, EPI>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    CG_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     configured[dev] = true;
   }
-  const int tiles = ((g.M + BM - 1) / BM) * (g.N / BN);
-  const int grid = tiles < cg_num_sms() ? tiles : cg_num_sms();
-  CG_CUDA(cg_launch_pdl(gemm_bf16_tn_kernel<BN, EPI>, dim3(grid), dim3(NUM_THREADS), smem, s, ta, tb, g));
+  const int tiles = ((g.M + CTAS * BM - 1) / (CTAS * BM)) * (g.N / BN);
+  int slots = cg_num_sms() / CTAS;  // CTAs, or CTA pairs
+  if (tiles < slots) slots = tiles;
+  CG_CUDA(cg_launch_pdl(kernel, dim3(CTAS * slots), dim3(NUM_THREADS), smem, s, ta, tb, g));
   return 0;
 }
 
-template <int BN>
+template <int BN, int CTAS>
 int dispatch(int epi, const CUtensorMap& ta, const CUtensorMap& tb, const GemmArgs& g, cudaStream_t s) {
   switch (epi) {
-    case CG_EPI_BIAS_BF16: return launch<BN, CG_EPI_BIAS_BF16>(ta, tb, g, s);
-    case CG_EPI_BIAS_RESID_F32: return launch<BN, CG_EPI_BIAS_RESID_F32>(ta, tb, g, s);
-    case CG_EPI_BIAS_QGELU_BF16: return launch<BN, CG_EPI_BIAS_QGELU_BF16>(ta, tb, g, s);
-    case CG_EPI_DQGELU_BF16: return launch<BN, CG_EPI_DQGELU_BF16>(ta, tb, g, s);
-    case CG_EPI_F32: return launch<BN, CG_EPI_F32>(ta, tb, g, s);
-    case CG_EPI_BF16: return launch<BN, CG_EPI_BF16>(ta, tb, g, s);
-    case CG_EPI_PATCH_POS_F32: return launch<BN, CG_EPI_PATCH_POS_F32>(ta, tb, g, s);
-  }
-  cg_set_error("cg_gemm_bf16_tn: unknown epilogue %d", epi);
-  return CG_EINVAL;
-}
-
-template <int EPI>
-int launch_pair(const CUtensorMap& ta, const CUtensorMap& tb, const GemmArgs& g, cudaStream_t s) {
-  constexpr size_t smem = (size_t)STAGES2 * (BM * BK * 2 + (BN2 / 2) * BK * 2) + 1024 + 256;
-  static bool configured[CG_MAX_DEVICES] = {};
-  const int dev = cg_device_index();
-  if (!configured[dev]) {
-    CG_CUDA(cudaFuncSetAttribute(gemm_bf16_tn_pair_kernel<EPI>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    configured[dev] = true;
-  }
-  const int tiles = ((g.M + 2 * BM - 1) / (2 * BM)) * (g.N / BN2);
-  int clusters = cg_num_sms() / 2;
-  if (tiles < clusters) clusters = tiles;
-  CG_CUDA(cg_launch_pdl(gemm_bf16_tn_pair_kernel<EPI>, dim3(2 * clusters), dim3(NUM_THREADS), smem, s, ta, tb, g));
-  return 0;
-}
-
-int dispatch_pair(int epi, const CUtensorMap& ta, const CUtensorMap& tb, const GemmArgs& g, cudaStream_t s) {
-  switch (epi) {
-    case CG_EPI_BIAS_BF16: return launch_pair<CG_EPI_BIAS_BF16>(ta, tb, g, s);
-    case CG_EPI_BIAS_RESID_F32: return launch_pair<CG_EPI_BIAS_RESID_F32>(ta, tb, g, s);
-    case CG_EPI_BIAS_QGELU_BF16: return launch_pair<CG_EPI_BIAS_QGELU_BF16>(ta, tb, g, s);
-    case CG_EPI_DQGELU_BF16: return launch_pair<CG_EPI_DQGELU_BF16>(ta, tb, g, s);
-    case CG_EPI_F32: return launch_pair<CG_EPI_F32>(ta, tb, g, s);
-    case CG_EPI_BF16: return launch_pair<CG_EPI_BF16>(ta, tb, g, s);
-    case CG_EPI_PATCH_POS_F32: return launch_pair<CG_EPI_PATCH_POS_F32>(ta, tb, g, s);
+    case CG_EPI_BIAS_BF16: return launch<BN, CTAS, CG_EPI_BIAS_BF16>(ta, tb, g, s);
+    case CG_EPI_BIAS_RESID_F32: return launch<BN, CTAS, CG_EPI_BIAS_RESID_F32>(ta, tb, g, s);
+    case CG_EPI_BIAS_QGELU_BF16: return launch<BN, CTAS, CG_EPI_BIAS_QGELU_BF16>(ta, tb, g, s);
+    case CG_EPI_DQGELU_BF16: return launch<BN, CTAS, CG_EPI_DQGELU_BF16>(ta, tb, g, s);
+    case CG_EPI_F32: return launch<BN, CTAS, CG_EPI_F32>(ta, tb, g, s);
+    case CG_EPI_BF16: return launch<BN, CTAS, CG_EPI_BF16>(ta, tb, g, s);
+    case CG_EPI_PATCH_POS_F32: return launch<BN, CTAS, CG_EPI_PATCH_POS_F32>(ta, tb, g, s);
   }
   cg_set_error("cg_gemm_bf16_tn: unknown epilogue %d", epi);
   return CG_EINVAL;
@@ -635,7 +531,7 @@ int choose_tile(int M, int N, int K, int epilogue) {
   const double c128 = waves(mt * (N / 128), sms) * 128.0 / (K > 1024 ? 0.75 : 0.85);  // the A tile is re-read for half the work: worse with long K
   const bool heavy_epi = epilogue == CG_EPI_BIAS_QGELU_BF16 || epilogue == CG_EPI_DQGELU_BF16;
   // a pair tile is two CTAs' worth of rows: per-SM cost = waves x 256 columns, ~10 % faster per tile when K is long
-  const double cpair = (can_pair && force_pair != 0 && !heavy_epi && K >= 1024) ? waves(mt2 * (N / BN2), sms / 2) * 256.0 / (K >= 2048 ? 1.10 : 1.02) : 1e30;
+  const double cpair = (can_pair && force_pair != 0 && !heavy_epi && K >= 1024) ? waves(mt2 * (N / 256), sms / 2) * 256.0 / (K >= 2048 ? 1.10 : 1.02) : 1e30;
   if (force_bn == 256) return cpair < c256 ? TILE_PAIR : TILE_256;
   if (cpair <= c256 && cpair <= c128) return TILE_PAIR;
   return c128 < c256 ? TILE_128 : TILE_256;
@@ -678,20 +574,15 @@ extern "C" int cg_gemm_bf16_tn(const void* A, const void* B, int M, int N, int K
                     (!aux || (((uintptr_t)aux & 31) == 0 && aux_row_bytes % 32 == 0)))
                        ? 1
                        : 0;
+  // the variant's <BN, CTAS>, and the rows of B one CTA stages, BN / CTAS
   const int tile = choose_tile(M, N, K, epilogue);
+  const auto run = tile == TILE_PAIR ? dispatch<256, 2> : tile == TILE_256 ? dispatch<256, 1> : dispatch<128, 1>;
+  const int b_rows = tile == TILE_256 ? 256 : 128;
   CUtensorMap ta, tb;
   int rc = cg_make_tensor_map_bf16(&ta, A, M, K, lda, BM);
   if (rc) return rc;
-  if (tile == TILE_PAIR) {
-    rc = cg_make_tensor_map_bf16(&tb, B, N, K, ldb, BN2 / 2);
-    if (rc) return rc;
-    GemmArgs gp = {M, N, K, bias, out, aux, (long long)ldo, pos, g2, wide};
-    return dispatch_pair(epilogue, ta, tb, gp, cg_stream(stream));
-  }
-  const int bn = tile == TILE_256 ? 256 : 128;
-  rc = cg_make_tensor_map_bf16(&tb, B, N, K, ldb, bn);
+  rc = cg_make_tensor_map_bf16(&tb, B, N, K, ldb, b_rows);
   if (rc) return rc;
-  GemmArgs g = {M, N, K, bias, out, aux, (long long)ldo, pos, g2, wide};
-  cudaStream_t s = cg_stream(stream);
-  return bn == 256 ? dispatch<256>(epilogue, ta, tb, g, s) : dispatch<128>(epilogue, ta, tb, g, s);
+  const GemmArgs g = {M, N, K, bias, out, aux, (long long)ldo, pos, g2, wide};
+  return run(epilogue, ta, tb, g, cg_stream(stream));
 }

@@ -22,6 +22,11 @@ EPI_DQGELU_BF16 = 3
 EPI_F32 = 4
 EPI_BF16 = 5
 EPI_PATCH_POS_F32 = 6
+# the ReLU-network epilogues, run through cg_gemm_bf16_tn_relu
+EPI_BIAS_RELU_BF16 = 7
+EPI_BIAS_RESID_RELU_BF16 = 8
+EPI_DRELU_BF16 = 9
+EPI_RESID_DRELU = 10
 
 GEMM_TILE_128x256 = 0
 GEMM_TILE_128x128 = 1
@@ -84,6 +89,14 @@ _SIGNATURES = {
     "cg_layernorm_bwd": (_I, [_P, _P, _P, _P, _P, _I, _I, _L, _I, _P, _P, _P]),
     "cg_gemm_bf16_tn": (_I, [_P, _P, _I, _I, _I, _L, _L, _I, _P, _P, _P, _L, _P, _I, _P]),
     "cg_gemm_tile_variant": (_I, [_I, _I, _I, _I]),
+    "cg_gemm_bf16_tn_relu": (_I, [_P, _P, _I, _I, _I, _L, _L, _I, _P, _P, _P, _P, _P, _L, _P]),
+    "cg_im2col3x3_nhwc": (_I, [_P, _I, _I, _I, _I, _L, _I, _I, _P, _P]),
+    "cg_conv3x3s2_dgrad": (_I, [_P, _I, _I, _I, _I, _L, _P, _I, _I, _P, _P]),
+    "cg_avgpool2x2_nhwc_fwd": (_I, [_P, _I, _I, _I, _I, _P, _P]),
+    "cg_avgpool2x2_nhwc_bwd": (_I, [_P, _I, _P, _I, _I, _I, _I, _P, _I, _P]),
+    "cg_resnet_attnpool_fwd": (_I, [_P, _P, _I, _I, _I, _P, _P]),
+    "cg_resnet_attnpool_bwd": (_I, [_P, _P, _I, _I, _I, _P, _P, _P]),
+    "cg_resnet_attnpool_dctx": (_I, [_P, _I, _I, _I, _P, _P]),
     "cg_attention_fwd": (_I, [_P, _I, _I, _I, _P, _P, _P]),
     "cg_attention_bwd": (_I, [_P, _P, _P, _P, _I, _I, _I, _P, _P, _P]),
     "cg_attention_causal_fwd": (_I, [_P, _I, _I, _I, _P, _P, _P]),

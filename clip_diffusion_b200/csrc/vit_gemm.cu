@@ -39,6 +39,10 @@ struct GemmArgs {
   const float* pos;
   int g2;
   int wide;  // rows of out / aux are 32-byte aligned: the epilogue may use 256-bit global accesses
+  // the ReLU-network epilogues (cg_gemm_bf16_tn_relu), addressed with ldo like out
+  const void* resid;  // bf16 (BIAS_RESID_RELU_BF16) or fp32 (RESID_DRELU, may alias out)
+  const void* mask;   // bf16 saved ReLU output (DRELU_BF16; RESID_DRELU when not NULL)
+  void* out_bf16;     // RESID_DRELU: bf16 copy of the fp32 out
 };
 
 using namespace tc;
@@ -128,7 +132,8 @@ __device__ __forceinline__ void epilogue_chunk(const GemmArgs& g, long long row,
   float v[32];
 #pragma unroll
   for (int j = 0; j < 32; ++j) v[j] = __uint_as_float(acc_u[j]);
-  if (EPI == CG_EPI_BIAS_BF16 || EPI == CG_EPI_BIAS_RESID_F32 || EPI == CG_EPI_BIAS_QGELU_BF16) {
+  if (EPI == CG_EPI_BIAS_BF16 || EPI == CG_EPI_BIAS_RESID_F32 || EPI == CG_EPI_BIAS_QGELU_BF16 || EPI == CG_EPI_BIAS_RELU_BF16 ||
+      EPI == CG_EPI_BIAS_RESID_RELU_BF16) {
     const float4* b4 = reinterpret_cast<const float4*>(g.bias + col);
 #pragma unroll
     for (int j = 0; j < 8; ++j) {
@@ -136,7 +141,45 @@ __device__ __forceinline__ void epilogue_chunk(const GemmArgs& g, long long row,
       v[4 * j] += b.x; v[4 * j + 1] += b.y; v[4 * j + 2] += b.z; v[4 * j + 3] += b.w;
     }
   }
-  if (EPI == CG_EPI_BIAS_RESID_F32 || EPI == CG_EPI_F32 || EPI == CG_EPI_PATCH_POS_F32) {
+  if (EPI == CG_EPI_BIAS_RELU_BF16 || EPI == CG_EPI_BIAS_RESID_RELU_BF16 || EPI == CG_EPI_DRELU_BF16 || EPI == CG_EPI_RESID_DRELU) {
+    // ReLU networks, as selects that follow torch: relu keeps a NaN (a NaN cutout stays visible to the step's NaN guard), and the
+    // derivative is threshold_backward's (zero where the saved output is <= 0, so an infinite accumulator under a zero mask gives 0)
+    const long long off = orow * g.ldo + col;
+    if (EPI == CG_EPI_BIAS_RESID_RELU_BF16) {
+      uint32_t w[16];
+      load_bf16x32(reinterpret_cast<const __nv_bfloat16*>(g.resid) + off, w, wide);
+#pragma unroll
+      for (int j = 0; j < 16; ++j) {
+        const __nv_bfloat162 p = *reinterpret_cast<const __nv_bfloat162*>(&w[j]);
+        v[2 * j] += __low2float(p);
+        v[2 * j + 1] += __high2float(p);
+      }
+    } else if (EPI == CG_EPI_RESID_DRELU) {
+      float r[32];
+      load_f32x32(reinterpret_cast<const float*>(g.resid) + off, r, wide);
+#pragma unroll
+      for (int j = 0; j < 32; ++j) v[j] += r[j];
+    }
+    if (EPI == CG_EPI_BIAS_RELU_BF16 || EPI == CG_EPI_BIAS_RESID_RELU_BF16) {
+#pragma unroll
+      for (int j = 0; j < 32; ++j) v[j] = v[j] < 0.f ? 0.f : v[j];
+    } else if (EPI == CG_EPI_DRELU_BF16 || g.mask) {
+      uint32_t w[16];
+      load_bf16x32(reinterpret_cast<const __nv_bfloat16*>(g.mask) + off, w, wide);
+#pragma unroll
+      for (int j = 0; j < 16; ++j) {
+        const __nv_bfloat162 p = *reinterpret_cast<const __nv_bfloat162*>(&w[j]);
+        v[2 * j] = __low2float(p) <= 0.f ? 0.f : v[2 * j];
+        v[2 * j + 1] = __high2float(p) <= 0.f ? 0.f : v[2 * j + 1];
+      }
+    }
+    if (EPI == CG_EPI_RESID_DRELU) {
+      store_f32x32(reinterpret_cast<float*>(g.out) + off, v, wide);
+      store_bf16x32(reinterpret_cast<__nv_bfloat16*>(g.out_bf16) + off, v, wide);
+    } else {
+      store_bf16x32(reinterpret_cast<__nv_bfloat16*>(g.out) + off, v, wide);
+    }
+  } else if (EPI == CG_EPI_BIAS_RESID_F32 || EPI == CG_EPI_F32 || EPI == CG_EPI_PATCH_POS_F32) {
     float* o = reinterpret_cast<float*>(g.out) + orow * g.ldo + col;
     if (EPI == CG_EPI_PATCH_POS_F32) {
       const float4* p4 = reinterpret_cast<const float4*>(g.pos + (1 + row % g.g2) * (long long)g.N + col);
@@ -497,6 +540,10 @@ int dispatch(int epi, const CUtensorMap& ta, const CUtensorMap& tb, const GemmAr
     case CG_EPI_F32: return launch<BN, CTAS, CG_EPI_F32>(ta, tb, g, s);
     case CG_EPI_BF16: return launch<BN, CTAS, CG_EPI_BF16>(ta, tb, g, s);
     case CG_EPI_PATCH_POS_F32: return launch<BN, CTAS, CG_EPI_PATCH_POS_F32>(ta, tb, g, s);
+    case CG_EPI_BIAS_RELU_BF16: return launch<BN, CTAS, CG_EPI_BIAS_RELU_BF16>(ta, tb, g, s);
+    case CG_EPI_BIAS_RESID_RELU_BF16: return launch<BN, CTAS, CG_EPI_BIAS_RESID_RELU_BF16>(ta, tb, g, s);
+    case CG_EPI_DRELU_BF16: return launch<BN, CTAS, CG_EPI_DRELU_BF16>(ta, tb, g, s);
+    case CG_EPI_RESID_DRELU: return launch<BN, CTAS, CG_EPI_RESID_DRELU>(ta, tb, g, s);
   }
   cg_set_error("cg_gemm_bf16_tn: unknown epilogue %d", epi);
   return CG_EINVAL;
@@ -544,36 +591,26 @@ extern "C" int cg_gemm_tile_variant(int M, int N, int K, int epilogue) {
   return choose_tile(M, N, K, epilogue);
 }
 
-extern "C" int cg_gemm_bf16_tn(const void* A, const void* B, int M, int N, int K, int64_t lda, int64_t ldb, int epilogue, const float* bias,
-                               void* out, void* aux, int64_t ldo, const float* pos, int g2, void* stream) {
-  CG_REQUIRE(A && B && out, "cg_gemm_bf16_tn: null operand");
-  CG_REQUIRE(M > 0 && N > 0 && K > 0, "cg_gemm_bf16_tn: bad sizes M=%d N=%d K=%d", M, N, K);
-  CG_REQUIRE(K % BK == 0, "cg_gemm_bf16_tn: K=%d must be a multiple of %d", K, BK);
-  CG_REQUIRE(N % 128 == 0, "cg_gemm_bf16_tn: N=%d must be a multiple of 128", N);
-  CG_REQUIRE(lda % 8 == 0 && ldb % 8 == 0 && lda >= K && ldb >= K, "cg_gemm_bf16_tn: leading dimensions must be >= K and multiples of 8");
-  CG_REQUIRE(((uintptr_t)A & 15) == 0 && ((uintptr_t)B & 15) == 0 && ((uintptr_t)out & 15) == 0, "cg_gemm_bf16_tn: pointers must be 16-byte aligned");
-  // the epilogue reads bias, aux and pos with 128-bit (or 256-bit) vector loads
-  CG_REQUIRE(((uintptr_t)bias & 15) == 0 && ((uintptr_t)aux & 15) == 0 && ((uintptr_t)pos & 15) == 0,
-             "cg_gemm_bf16_tn: bias, aux and pos must be 16-byte aligned");
-  CG_REQUIRE(ldo % 8 == 0 && ldo >= N, "cg_gemm_bf16_tn: ldo=%lld must be >= N and a multiple of 8", (long long)ldo);
-  const bool needs_bias = epilogue == CG_EPI_BIAS_BF16 || epilogue == CG_EPI_BIAS_RESID_F32 || epilogue == CG_EPI_BIAS_QGELU_BF16;
-  CG_REQUIRE(!needs_bias || bias, "cg_gemm_bf16_tn: epilogue %d needs a bias", epilogue);
-  CG_REQUIRE((epilogue != CG_EPI_BIAS_QGELU_BF16 && epilogue != CG_EPI_DQGELU_BF16 && epilogue != CG_EPI_BIAS_RESID_F32) || aux, "cg_gemm_bf16_tn: epilogue %d needs aux", epilogue);
-  CG_REQUIRE(epilogue != CG_EPI_PATCH_POS_F32 || (pos && g2 > 0 && M % g2 == 0), "cg_gemm_bf16_tn: patch epilogue needs pos and g2 | M");
-  // 256-bit epilogue accesses: every row start of out (and aux) must be 32-byte aligned.  Element size: fp32 outputs 4, bf16 2;
-  // aux is fp32 for the residual epilogue, bf16 for the QuickGELU ones.  CG_GEMM_WIDE=0 forces the 128-bit path.
-  static int wide_env = -1;
-  if (wide_env < 0) {
-    const char* e = getenv("CG_GEMM_WIDE");
-    wide_env = (e && atoi(e) == 0) ? 0 : 1;
-  }
-  const bool out_f32 = epilogue == CG_EPI_BIAS_RESID_F32 || epilogue == CG_EPI_F32 || epilogue == CG_EPI_PATCH_POS_F32;
-  const long long row_bytes = (long long)ldo * (out_f32 ? 4 : 2);
-  const long long aux_row_bytes = (long long)ldo * (epilogue == CG_EPI_BIAS_RESID_F32 ? 4 : 2);
-  const int wide = (wide_env && epilogue != CG_EPI_PATCH_POS_F32 && ((uintptr_t)out & 31) == 0 && row_bytes % 32 == 0 &&
-                    (!aux || (((uintptr_t)aux & 31) == 0 && aux_row_bytes % 32 == 0)))
-                       ? 1
-                       : 0;
+namespace {
+
+// 256-bit epilogue accesses need every row start of out (and of each array the epilogue reads with out's ldo) 32-byte aligned.
+// CG_GEMM_WIDE=0 forces the 128-bit path.
+bool wide_enabled() {
+  static const int wide_env = env_choice("CG_GEMM_WIDE");
+  return wide_env != 0;
+}
+bool rows32(const void* p, long long ldo, int elem_bytes) { return !p || (((uintptr_t)p & 31) == 0 && ldo * elem_bytes % 32 == 0); }
+
+// the checks both entry points share, then the launch on the tile variant chosen for the problem
+int run_gemm(const char* fn, const void* A, const void* B, int64_t lda, int64_t ldb, int epilogue, const GemmArgs& g, void* stream) {
+  const int M = g.M, N = g.N, K = g.K;
+  CG_REQUIRE(A && B && g.out, "%s: null operand", fn);
+  CG_REQUIRE(M > 0 && N > 0 && K > 0, "%s: bad sizes M=%d N=%d K=%d", fn, M, N, K);
+  CG_REQUIRE(K % BK == 0, "%s: K=%d must be a multiple of %d", fn, K, BK);
+  CG_REQUIRE(N % 128 == 0, "%s: N=%d must be a multiple of 128", fn, N);
+  CG_REQUIRE(lda % 8 == 0 && ldb % 8 == 0 && lda >= K && ldb >= K, "%s: leading dimensions must be >= K and multiples of 8", fn);
+  CG_REQUIRE(((uintptr_t)A & 15) == 0 && ((uintptr_t)B & 15) == 0 && ((uintptr_t)g.out & 15) == 0, "%s: pointers must be 16-byte aligned", fn);
+  CG_REQUIRE(g.ldo % 8 == 0 && g.ldo >= N, "%s: ldo=%lld must be >= N and a multiple of 8", fn, g.ldo);
   // the variant's <BN, CTAS>, and the rows of B one CTA stages, BN / CTAS
   const int tile = choose_tile(M, N, K, epilogue);
   const auto run = tile == TILE_PAIR ? dispatch<256, 2> : tile == TILE_256 ? dispatch<256, 1> : dispatch<128, 1>;
@@ -583,6 +620,45 @@ extern "C" int cg_gemm_bf16_tn(const void* A, const void* B, int M, int N, int K
   if (rc) return rc;
   rc = cg_make_tensor_map_bf16(&tb, B, N, K, ldb, b_rows);
   if (rc) return rc;
-  const GemmArgs g = {M, N, K, bias, out, aux, (long long)ldo, pos, g2, wide};
   return run(epilogue, ta, tb, g, cg_stream(stream));
+}
+
+}  // namespace
+
+extern "C" int cg_gemm_bf16_tn(const void* A, const void* B, int M, int N, int K, int64_t lda, int64_t ldb, int epilogue, const float* bias,
+                               void* out, void* aux, int64_t ldo, const float* pos, int g2, void* stream) {
+  CG_REQUIRE(epilogue >= 0 && epilogue <= CG_EPI_PATCH_POS_F32, "cg_gemm_bf16_tn: unknown epilogue %d (the ReLU epilogues run through cg_gemm_bf16_tn_relu)",
+             epilogue);
+  // the epilogue reads bias, aux and pos with 128-bit (or 256-bit) vector loads
+  CG_REQUIRE(((uintptr_t)bias & 15) == 0 && ((uintptr_t)aux & 15) == 0 && ((uintptr_t)pos & 15) == 0,
+             "cg_gemm_bf16_tn: bias, aux and pos must be 16-byte aligned");
+  const bool needs_bias = epilogue == CG_EPI_BIAS_BF16 || epilogue == CG_EPI_BIAS_RESID_F32 || epilogue == CG_EPI_BIAS_QGELU_BF16;
+  CG_REQUIRE(!needs_bias || bias, "cg_gemm_bf16_tn: epilogue %d needs a bias", epilogue);
+  CG_REQUIRE((epilogue != CG_EPI_BIAS_QGELU_BF16 && epilogue != CG_EPI_DQGELU_BF16 && epilogue != CG_EPI_BIAS_RESID_F32) || aux, "cg_gemm_bf16_tn: epilogue %d needs aux", epilogue);
+  CG_REQUIRE(epilogue != CG_EPI_PATCH_POS_F32 || (pos && g2 > 0 && M % g2 == 0), "cg_gemm_bf16_tn: patch epilogue needs pos and g2 | M");
+  // element size: fp32 outputs 4, bf16 2; aux is fp32 for the residual epilogue, bf16 for the QuickGELU ones
+  const bool out_f32 = epilogue == CG_EPI_BIAS_RESID_F32 || epilogue == CG_EPI_F32 || epilogue == CG_EPI_PATCH_POS_F32;
+  const int wide = wide_enabled() && epilogue != CG_EPI_PATCH_POS_F32 && out && rows32(out, ldo, out_f32 ? 4 : 2) &&
+                   rows32(aux, ldo, epilogue == CG_EPI_BIAS_RESID_F32 ? 4 : 2);
+  GemmArgs g = {M, N, K, bias, out, aux, (long long)ldo, pos, g2, wide, nullptr, nullptr, nullptr};
+  return run_gemm("cg_gemm_bf16_tn", A, B, lda, ldb, epilogue, g, stream);
+}
+
+extern "C" int cg_gemm_bf16_tn_relu(const void* A, const void* B, int M, int N, int K, int64_t lda, int64_t ldb, int epilogue, const float* bias,
+                                    const void* resid, const void* mask, void* out, void* out_bf16, int64_t ldo, void* stream) {
+  CG_REQUIRE(epilogue >= CG_EPI_BIAS_RELU_BF16 && epilogue <= CG_EPI_RESID_DRELU, "cg_gemm_bf16_tn_relu: epilogue %d is not a ReLU epilogue", epilogue);
+  const bool has_bias = epilogue == CG_EPI_BIAS_RELU_BF16 || epilogue == CG_EPI_BIAS_RESID_RELU_BF16;
+  const bool has_resid = epilogue == CG_EPI_BIAS_RESID_RELU_BF16 || epilogue == CG_EPI_RESID_DRELU;
+  CG_REQUIRE(has_bias == (bias != nullptr), "cg_gemm_bf16_tn_relu: epilogue %d %s a bias", epilogue, has_bias ? "needs" : "takes no");
+  CG_REQUIRE(has_resid == (resid != nullptr), "cg_gemm_bf16_tn_relu: epilogue %d %s a residual", epilogue, has_resid ? "needs" : "takes no");
+  CG_REQUIRE(epilogue != CG_EPI_DRELU_BF16 || mask, "cg_gemm_bf16_tn_relu: DRELU_BF16 needs a mask");
+  CG_REQUIRE(epilogue == CG_EPI_DRELU_BF16 || epilogue == CG_EPI_RESID_DRELU || !mask, "cg_gemm_bf16_tn_relu: epilogue %d takes no mask", epilogue);
+  CG_REQUIRE((epilogue == CG_EPI_RESID_DRELU) == (out_bf16 != nullptr), "cg_gemm_bf16_tn_relu: out_bf16 is RESID_DRELU's second output (and only its)");
+  CG_REQUIRE(((uintptr_t)bias & 15) == 0 && ((uintptr_t)resid & 15) == 0 && ((uintptr_t)mask & 15) == 0 && ((uintptr_t)out_bf16 & 15) == 0,
+             "cg_gemm_bf16_tn_relu: bias, resid, mask and out_bf16 must be 16-byte aligned");
+  const bool f32 = epilogue == CG_EPI_RESID_DRELU;  // out and resid are fp32
+  const int wide = wide_enabled() && out && rows32(out, ldo, f32 ? 4 : 2) && rows32(resid, ldo, f32 ? 4 : 2) && rows32(mask, ldo, 2) &&
+                   rows32(out_bf16, ldo, 2);
+  GemmArgs g = {M, N, K, bias, out, nullptr, (long long)ldo, nullptr, 0, wide, resid, mask, out_bf16};
+  return run_gemm("cg_gemm_bf16_tn_relu", A, B, lda, ldb, epilogue, g, stream);
 }

@@ -12,6 +12,10 @@ reference gets from the un-vendored ``clip`` package -- is implemented here on t
   backward               dgrad only: the towers are frozen (models.py:67-71), so every backward GEMM is
                          activation-gradient x pre-transposed weight, packed once at load
 
+OpenAI's ModifiedResNet image tower (RN101, the fourth of Config.chosen_clip_models) runs on the same GEMM with ReLU-network
+epilogues: NHWC bf16 activations, BatchNorm folded at load, 3x3 convolutions as im2col + GEMM, the attention pool on the ViT's
+attention kernels.  It has the ViT tower's interface (patch 1: the cutout kernel's NHWC image), so the guidance step drives both alike.
+
 ``model.encode_text(tokens)`` (utils/functional.py:91-94, once per job) runs OpenAI's text transformer on the same kernels with
 a causal attention forward; that tower is built on its first call.
 
@@ -25,7 +29,7 @@ import torch
 from torch import nn
 
 from clip_diffusion_b200 import _lib
-from clip_diffusion_b200.vit_ops import gemm_bf16_tn
+from clip_diffusion_b200.vit_ops import gemm_bf16_tn, gemm_bf16_tn_relu
 
 # name: (input_resolution, patch, width, layers, heads, embed_dim)     E as in models.py:33-37
 CLIP_CONFIGS = {
@@ -42,6 +46,12 @@ CLIP_TEXT_CONFIGS = {
     "ViT-B/16": (77, 49408, 512, 12, 8, 512),
     "ViT-L/14": (77, 49408, 768, 12, 12, 768),
     "ViT-L/14@336px": (77, 49408, 768, 12, 12, 768),
+    "RN101": (77, 49408, 512, 12, 8, 512),
+}
+
+# name: (input_resolution, layers, width, heads, embed_dim) of OpenAI's ModifiedResNet (build_model infers them from the state dict)
+CLIP_RESNET_CONFIGS = {
+    "RN101": (224, (3, 4, 23, 3), 64, 32, 512),
 }
 
 
@@ -71,6 +81,16 @@ def register_clip_text_config(name, context, vocab, width, layers, heads, embed_
     if not 0 < context <= _lib.ATTN_TC_MAX_T:
         raise ValueError("the context length must lie in [1, %d]" % _lib.ATTN_TC_MAX_T)
     CLIP_TEXT_CONFIGS[name] = (context, vocab, width, layers, heads, embed_dim)
+
+
+def register_clip_resnet_config(name, input_resolution, layers, width, heads, embed_dim):
+    """Extra ModifiedResNet shapes (tests use tiny ones).  The attention pool's width 32*width must equal heads*64; its T = (res/32)^2 + 1
+    is at most _lib.ATTN_TC_MAX_T; embed_dim (the N of the c_proj GEMM) is a multiple of 128."""
+    if len(layers) != 4 or min(layers) < 1 or input_resolution % 32 or width % 2:
+        raise ValueError("a ModifiedResNet has four stages of >= 1 block, an input resolution divisible by 32 and an even width")
+    if 32 * width != 64 * heads or embed_dim % 128 or (input_resolution // 32) ** 2 + 1 > _lib.ATTN_TC_MAX_T:
+        raise ValueError("the attention pool needs 32*width == heads*64, embed_dim % 128 == 0 and (res/32)^2 + 1 <= %d" % _lib.ATTN_TC_MAX_T)
+    CLIP_RESNET_CONFIGS[name] = (input_resolution, tuple(layers), width, heads, embed_dim)
 
 
 def random_clip_state_dict(name, seed=1):
@@ -191,30 +211,13 @@ def _block_forward(attention, blk, n, T, heads, x, out, L, h, hg):
     gemm_bf16_tn(hg, blk["w_proj"], _lib.EPI_BIAS_RESID_F32, bias=blk["b_proj"], out=out, aux=L["x_mid"])
 
 
-class VisionTransformerB200:
-    """Frozen OpenAI-style CLIP vision transformer: forward + input-gradient backward on sm_100a kernels."""
+class _GraphTower:
+    """What the image towers share: the interface the guidance step and _EncodeImageFn use (input_resolution, patch, kpad, grid,
+    output_dim, forward_patches, backward_patches), per-batch-size workspaces with stable addresses, the generation id that makes a
+    stale backward an error, and CUDA-graph passes.  A subclass sets those attributes and provides _new_workspace(n) (its activation
+    buffers), _forward_body(ws, n) (patches -> emb) and _backward_body(ws, n) (demb -> dpatch)."""
 
-    def __init__(self, name, state_dict, device):
-        res, patch, width, layers, heads, embed = CLIP_CONFIGS[name]
-        self.name = name
-        self.input_resolution, self.patch, self.width, self.layers, self.heads, self.output_dim = res, patch, width, layers, heads, embed
-        self.grid = res // patch
-        self.tokens = self.grid ** 2 + 1
-        self.kdim = 3 * patch * patch
-        self.kpad = (self.kdim + 127) // 128 * 128  # K of the patch GEMM (x64) and N of its dgrad (x128)
-        self.device = torch.device(device)
-        sd, dev = state_dict, self.device
-        w = sd["visual.conv1.weight"].reshape(width, self.kdim)
-        wpad = torch.zeros(width, self.kpad)
-        wpad[:, : self.kdim] = w
-        self.w_patch = _bf16(wpad, dev)          # [D, Kpad]   fwd  B operand
-        self.w_patch_t = _bf16(wpad.t(), dev)    # [Kpad, D]   dgrad B operand
-        self.cls = _f32(sd["visual.class_embedding"], dev)
-        self.pos = _f32(sd["visual.positional_embedding"], dev)
-        self.ln_pre = (_f32(sd["visual.ln_pre.weight"], dev), _f32(sd["visual.ln_pre.bias"], dev))
-        self.ln_post = (_f32(sd["visual.ln_post.weight"], dev), _f32(sd["visual.ln_post.bias"], dev))
-        self.proj = _f32(sd["visual.proj"], dev)
-        self.blocks = _pack_blocks(sd, "visual.transformer.resblocks.", layers, dev, transposed=True)
+    def _init_graph_tower(self):
         self._ws = {}  # persistent activation workspaces per batch size (stable addresses => TMA descriptor cache hits)
         self._generation = 0  # bumped by every forward: the saved activations live in the shared workspace, not in an autograd ctx
         # CUDA graphs: a tower pass is ~7 C-ABI calls per layer and direction on fixed buffers; issuing them one by one costs the host
@@ -228,26 +231,16 @@ class VisionTransformerB200:
         ws = self._ws.get(n)
         if ws is not None:
             return ws
-        dev, D, T, M = self.device, self.width, self.tokens, n * self.tokens
-        f32 = lambda *s: torch.empty(*s, device=dev, dtype=torch.float32)
-        b16 = lambda *s: torch.empty(*s, device=dev, dtype=torch.bfloat16)
-        ws = {
-            "x0": f32(M, D), "mean0": f32(M), "rstd0": f32(M),
-            "h": b16(M, D), "hg": b16(M, 4 * D),
-            "layers": [
-                {"x_in": f32(M, D), "mean1": f32(M), "rstd1": f32(M), "qkv": b16(M, 3 * D), "ctx": b16(M, D), "lse": f32(n, self.heads, T),
-                 "x_mid": f32(M, D), "mean2": f32(M), "rstd2": f32(M), "u": b16(M, 4 * D)}
-                for _ in range(self.layers)
-            ],
-            "x_out": f32(M, D), "meanp": f32(n), "rstdp": f32(n), "y": f32(n, D),
-            # backward
-            "dx": f32(M, D), "dxb": b16(M, D), "dy": f32(n, D), "du": b16(M, 4 * D), "dh": f32(M, D), "dctx": b16(M, D),
-            "dqkv": b16(M, 3 * D), "delta": f32(n, self.heads, T), "dx0": f32(M, D), "dtok": b16(n * (T - 1), D),
-            # static input / output buffers of the (graph-replayable) passes
-            "patches": b16(n, self.grid ** 2, self.kpad), "emb": f32(n, self.output_dim), "demb": f32(n, self.output_dim),
-            "dpatch": f32(n, self.grid ** 2, self.kpad),
+        dev = self.device
+        ws = self._new_workspace(n)
+        # static input / output buffers of the (graph-replayable) passes
+        ws.update({
+            "patches": torch.empty(n, self.grid ** 2, self.kpad, device=dev, dtype=torch.bfloat16),
+            "emb": torch.empty(n, self.output_dim, device=dev, dtype=torch.float32),
+            "demb": torch.empty(n, self.output_dim, device=dev, dtype=torch.float32),
+            "dpatch": torch.empty(n, self.grid ** 2, self.kpad, device=dev, dtype=torch.float32),
             "graphs": {},
-        }
+        })
         if len(self._ws) >= 4:  # bound the footprint when batch sizes keep changing (cut schedules)
             self._ws.pop(next(iter(self._ws)))
         self._ws[n] = ws
@@ -257,8 +250,7 @@ class VisionTransformerB200:
     def forward_patches(self, patches):
         """patches: [N, g*g, Kpad] bf16 im2col rows of the (CLIP-normalised) images -> embeddings [N, E] fp32."""
         n = patches.shape[0]
-        g2, D, T, E = self.grid ** 2, self.width, self.tokens, self.output_dim
-        M = n * T
+        g2 = self.grid ** 2
         if patches.shape[1] != g2 or patches.shape[2] != self.kpad or patches.dtype != torch.bfloat16:
             raise ValueError("expected bf16 patches of shape [N, %d, %d], got %s %s" % (g2, self.kpad, tuple(patches.shape), patches.dtype))
         ws = self._workspace(n)
@@ -304,22 +296,6 @@ class VisionTransformerB200:
         _lib.kernel_launches += st["launches"]
         _lib.launch_count += st["calls_per_pass"]
 
-    def _forward_body(self, ws, n):
-        g2, D, T, E = self.grid ** 2, self.width, self.tokens, self.output_dim
-        M = n * T
-        P, C = _lib.ptr, _lib.call
-        a = ws["patches"].view(n * g2, self.kpad)
-        gemm_bf16_tn(a, self.w_patch, _lib.EPI_PATCH_POS_F32, out=ws["x0"], pos=self.pos, g2=g2)
-        C("cg_vit_set_cls_rows", P(self.cls), P(self.pos), n, T, D, P(ws["x0"]))
-        x = ws["layers"][0]["x_in"] if self.layers else ws["x_out"]
-        C("cg_layernorm_fwd", P(ws["x0"]), P(self.ln_pre[0]), P(self.ln_pre[1]), M, D, D, None, P(x), P(ws["mean0"]), P(ws["rstd0"]))
-        for i, (blk, L) in enumerate(zip(self.blocks, ws["layers"])):
-            x_next = ws["layers"][i + 1]["x_in"] if i + 1 < self.layers else ws["x_out"]
-            _block_forward("cg_attention_fwd", blk, n, T, self.heads, L["x_in"], x_next, L, ws["h"], ws["hg"])
-        # ln_post on the class-token rows (row stride T*D), then the projection
-        C("cg_layernorm_fwd", P(ws["x_out"]), P(self.ln_post[0]), P(self.ln_post[1]), n, D, T * D, None, P(ws["y"]), P(ws["meanp"]), P(ws["rstdp"]))
-        C("cg_vit_proj_fwd", P(ws["y"]), P(self.proj), n, D, E, P(ws["emb"]))
-
     # ------------------------------------------------------------------ backward (input gradient only)
     def backward_patches(self, demb, generation=None):
         """demb [N, E] fp32 -> d(patches) [N, g*g, Kpad] fp32, for the activations of the latest forward.  The saved activations
@@ -344,6 +320,68 @@ class VisionTransformerB200:
         # the gradient buffer belongs to the workspace: consume it before the next backward of the same batch size (sample.py does)
         return ws["dpatch"]
 
+
+class VisionTransformerB200(_GraphTower):
+    """Frozen OpenAI-style CLIP vision transformer: forward + input-gradient backward on sm_100a kernels."""
+
+    def __init__(self, name, state_dict, device):
+        res, patch, width, layers, heads, embed = CLIP_CONFIGS[name]
+        self.name = name
+        self.input_resolution, self.patch, self.width, self.layers, self.heads, self.output_dim = res, patch, width, layers, heads, embed
+        self.grid = res // patch
+        self.tokens = self.grid ** 2 + 1
+        self.kdim = 3 * patch * patch
+        self.kpad = (self.kdim + 127) // 128 * 128  # K of the patch GEMM (x64) and N of its dgrad (x128)
+        self.device = torch.device(device)
+        sd, dev = state_dict, self.device
+        w = sd["visual.conv1.weight"].reshape(width, self.kdim)
+        wpad = torch.zeros(width, self.kpad)
+        wpad[:, : self.kdim] = w
+        self.w_patch = _bf16(wpad, dev)          # [D, Kpad]   fwd  B operand
+        self.w_patch_t = _bf16(wpad.t(), dev)    # [Kpad, D]   dgrad B operand
+        self.cls = _f32(sd["visual.class_embedding"], dev)
+        self.pos = _f32(sd["visual.positional_embedding"], dev)
+        self.ln_pre = (_f32(sd["visual.ln_pre.weight"], dev), _f32(sd["visual.ln_pre.bias"], dev))
+        self.ln_post = (_f32(sd["visual.ln_post.weight"], dev), _f32(sd["visual.ln_post.bias"], dev))
+        self.proj = _f32(sd["visual.proj"], dev)
+        self.blocks = _pack_blocks(sd, "visual.transformer.resblocks.", layers, dev, transposed=True)
+        self._init_graph_tower()
+
+    def _new_workspace(self, n):
+        dev, D, T, M = self.device, self.width, self.tokens, n * self.tokens
+        f32 = lambda *s: torch.empty(*s, device=dev, dtype=torch.float32)
+        b16 = lambda *s: torch.empty(*s, device=dev, dtype=torch.bfloat16)
+        return {
+            "x0": f32(M, D), "mean0": f32(M), "rstd0": f32(M),
+            "h": b16(M, D), "hg": b16(M, 4 * D),
+            "layers": [
+                {"x_in": f32(M, D), "mean1": f32(M), "rstd1": f32(M), "qkv": b16(M, 3 * D), "ctx": b16(M, D), "lse": f32(n, self.heads, T),
+                 "x_mid": f32(M, D), "mean2": f32(M), "rstd2": f32(M), "u": b16(M, 4 * D)}
+                for _ in range(self.layers)
+            ],
+            "x_out": f32(M, D), "meanp": f32(n), "rstdp": f32(n), "y": f32(n, D),
+            # backward
+            "dx": f32(M, D), "dxb": b16(M, D), "dy": f32(n, D), "du": b16(M, 4 * D), "dh": f32(M, D), "dctx": b16(M, D),
+            "dqkv": b16(M, 3 * D), "delta": f32(n, self.heads, T), "dx0": f32(M, D), "dtok": b16(n * (T - 1), D),
+        }
+
+    def _forward_body(self, ws, n):
+        g2, D, T, E = self.grid ** 2, self.width, self.tokens, self.output_dim
+        M = n * T
+        P, C = _lib.ptr, _lib.call
+        a = ws["patches"].view(n * g2, self.kpad)
+        gemm_bf16_tn(a, self.w_patch, _lib.EPI_PATCH_POS_F32, out=ws["x0"], pos=self.pos, g2=g2)
+        C("cg_vit_set_cls_rows", P(self.cls), P(self.pos), n, T, D, P(ws["x0"]))
+        x = ws["layers"][0]["x_in"] if self.layers else ws["x_out"]
+        C("cg_layernorm_fwd", P(ws["x0"]), P(self.ln_pre[0]), P(self.ln_pre[1]), M, D, D, None, P(x), P(ws["mean0"]), P(ws["rstd0"]))
+        for i, (blk, L) in enumerate(zip(self.blocks, ws["layers"])):
+            x_next = ws["layers"][i + 1]["x_in"] if i + 1 < self.layers else ws["x_out"]
+            _block_forward("cg_attention_fwd", blk, n, T, self.heads, L["x_in"], x_next, L, ws["h"], ws["hg"])
+        # ln_post on the class-token rows (row stride T*D), then the projection
+        C("cg_layernorm_fwd", P(ws["x_out"]), P(self.ln_post[0]), P(self.ln_post[1]), n, D, T * D, None, P(ws["y"]), P(ws["meanp"]), P(ws["rstdp"]))
+        C("cg_vit_proj_fwd", P(ws["y"]), P(self.proj), n, D, E, P(ws["emb"]))
+
+    # ------------------------------------------------------------------ backward (input gradient only)
     def _backward_body(self, ws, n):
         g2, D, T, E = self.grid ** 2, self.width, self.tokens, self.output_dim
         M = n * T
@@ -371,6 +409,321 @@ class VisionTransformerB200:
         patch = 2 * (T - 1) * self.kdim * D + 2 * D * E
         fwd = 24 * T * D * D * L + 4 * T * T * D * L + patch
         bwd = 24 * T * D * D * L + 8 * T * T * D * L + patch
+        return n * (fwd + bwd)
+
+
+# ---------------------------------------------------------------------------------------------------------------------- ModifiedResNet
+_BN_LEAVES = ("weight", "bias", "running_mean", "running_var", "num_batches_tracked")
+BN_EPS = 1e-5
+
+
+def _resnet_blocks(name):
+    """(prefix, inplanes, planes, stride, downsample) of every Bottleneck, in order (OpenAI ModifiedResNet._make_layer)."""
+    _, layers, width, _, _ = CLIP_RESNET_CONFIGS[name]
+    blocks, inplanes = [], width
+    for li, nb in enumerate(layers):
+        planes, stride = width * 2 ** li, 1 if li == 0 else 2
+        for i in range(nb):
+            s = stride if i == 0 else 1
+            blocks.append(("visual.layer%d.%d." % (li + 1, i), inplanes, planes, s, s > 1 or inplanes != 4 * planes))
+            inplanes = 4 * planes
+    return blocks
+
+
+def clip_resnet_state_dict_shapes(name):
+    """{key: shape} of the ``visual.*`` tensors of an OpenAI ModifiedResNet CLIP, in the order of OpenAI's state dict."""
+    res, _, width, _, embed = CLIP_RESNET_CONFIGS[name]
+    shapes = {}
+
+    def conv_bn(conv, bn, cout, cin, k):
+        shapes[conv + ".weight"] = (cout, cin, k, k)
+        shapes.update((bn + "." + leaf, () if leaf == "num_batches_tracked" else (cout,)) for leaf in _BN_LEAVES)
+
+    for i, (cout, cin) in enumerate(((width // 2, 3), (width // 2, width // 2), (width, width // 2))):
+        conv_bn("visual.conv%d" % (i + 1), "visual.bn%d" % (i + 1), cout, cin, 3)
+    for p, cin, planes, _, ds in _resnet_blocks(name):
+        conv_bn(p + "conv1", p + "bn1", planes, cin, 1)
+        conv_bn(p + "conv2", p + "bn2", planes, planes, 3)
+        conv_bn(p + "conv3", p + "bn3", 4 * planes, planes, 1)
+        if ds:
+            conv_bn(p + "downsample.0", p + "downsample.1", 4 * planes, cin, 1)
+    C = 32 * width
+    shapes["visual.attnpool.positional_embedding"] = ((res // 32) ** 2 + 1, C)
+    for proj in ("k_proj", "q_proj", "v_proj"):
+        shapes["visual.attnpool.%s.weight" % proj], shapes["visual.attnpool.%s.bias" % proj] = (C, C), (C,)
+    shapes["visual.attnpool.c_proj.weight"], shapes["visual.attnpool.c_proj.bias"] = (embed, C), (embed,)
+    return shapes
+
+
+def random_clip_resnet_state_dict(name, seed=1):
+    """Random weights with the keys and shapes of OpenAI's ModifiedResNet ``visual.*`` tensors, chosen so that signal crosses every
+    block: He-scaled convolutions, BatchNorm statistics and affines perturbed away from the identity, and a small bn3 gamma (~0.25)
+    so that each Bottleneck's branch adds to its identity without swamping it (OpenAI's zero bn3 gamma would make every block an
+    identity).  The attention pool follows OpenAI's initialize_parameters (std C^-1/2), with biases perturbed away from 0."""
+    g = torch.Generator().manual_seed(seed)
+    n = lambda *s: torch.randn(*s, generator=g)
+    sd = {}
+    for k, shape in clip_resnet_state_dict_shapes(name).items():
+        leaf = k.rsplit(".", 1)[-1]
+        bn3 = ".bn3." in k
+        if k.endswith("num_batches_tracked"):
+            sd[k] = torch.tensor(0, dtype=torch.long)
+        elif k.startswith("visual.attnpool."):
+            C = shape[-1]
+            sd[k] = C ** -0.5 * n(*shape) if leaf in ("weight", "positional_embedding") else 0.02 * n(*shape)
+        elif len(shape) == 4:
+            sd[k] = math.sqrt(2.0 / (shape[1] * shape[2] * shape[3])) * n(*shape)
+        elif leaf == "weight":
+            sd[k] = (0.25 if bn3 else 1.0) * (1 + 0.1 * n(*shape))
+        elif leaf == "bias":
+            sd[k] = (0.025 if bn3 else 0.1) * n(*shape)
+        elif leaf == "running_mean":
+            sd[k] = 0.1 * n(*shape)
+        else:
+            sd[k] = 1 + 0.2 * torch.rand(*shape, generator=g)
+    return sd
+
+
+def fold_batchnorm(weight, bn_weight, bn_bias, running_mean, running_var, eps=BN_EPS):
+    """conv (no bias) followed by eval-mode BatchNorm as one convolution with bias, in float64:
+    w' = w gamma / sqrt(var + eps), b' = beta - mean gamma / sqrt(var + eps)."""
+    s = bn_weight.double() / torch.sqrt(running_var.double() + eps)
+    return weight.double() * s.view(-1, *([1] * (weight.dim() - 1))), bn_bias.double() - running_mean.double() * s
+
+
+def _r128(c):
+    return (c + 127) // 128 * 128
+
+
+def _r64(c):
+    return (c + 63) // 64 * 64
+
+
+def _padded(w, rows, cols):
+    out = torch.zeros(rows, cols, dtype=w.dtype)
+    out[: w.shape[0], : w.shape[1]] = w
+    return out
+
+
+def _resnet_device(device):
+    device = torch.device(device)
+    if device.type != "cuda":
+        raise ValueError("the ModifiedResNet CLIP tower runs on a CUDA device only (got %s): it has no CPU path" % device)
+    return device
+
+
+class _Conv:
+    """One convolution with its BatchNorm folded in, packed at load as the B operands of its GEMMs (bf16, channel counts padded:
+    N to 128, K to 64, with zero rows / columns): ``w`` [cout', K] for the forward, ``b`` [cout'] fp32 its folded bias, ``wt`` the
+    input gradient's operand -- W^T [cin', K(cout)] for a 1x1 convolution, the flipped W'[cin', (ky, kx, cout)] for a 3x3 one."""
+
+    def __init__(self, sd, conv, bn, device, dgrad=True):
+        w, b = fold_batchnorm(sd[conv + ".weight"], *(sd[bn + "." + leaf] for leaf in _BN_LEAVES[:4]))
+        w = w.to(torch.bfloat16).double()  # the one rounding of the folded weights; every operand below is exact in bf16
+        self.cout, self.cin, k = w.shape[0], w.shape[1], w.shape[2]
+        self.k = _r64(k * k * self.cin)  # GEMM K of the forward
+        self.w = _bf16(_padded(w.permute(0, 2, 3, 1).reshape(self.cout, -1), _r128(self.cout), self.k), device)
+        self.b = _f32(_padded(b.view(-1, 1), _r128(self.cout), 1).view(-1), device)
+        self.kt = _r64(k * k * self.cout)  # GEMM K of the input gradient
+        if dgrad and k == 1:
+            self.wt = _bf16(_padded(w.view(self.cout, self.cin).t(), _r128(self.cin), self.kt), device)
+        elif dgrad:
+            self.wt = _bf16(_padded(w.flip(2, 3).permute(1, 2, 3, 0).reshape(self.cin, -1), _r128(self.cin), self.kt), device)
+        self.w_f32 = w  # host copy (the stem's stride-2 dgrad reads it as fp32)
+
+
+class ModifiedResNetB200(_GraphTower):
+    """Frozen OpenAI CLIP ModifiedResNet (the RN image towers): forward + input-gradient backward on sm_100a kernels.  Activations are
+    NHWC bf16 rows with channel counts padded to 128 (zero channels); BatchNorm is folded into the convolutions; each 3x3 convolution is
+    cg_im2col3x3_nhwc + a GEMM, the ReLUs, residuals and ReLU derivatives live in the GEMM epilogues.  The gradient's residual stream
+    is fp32 with a bf16 copy as the next GEMM's operand.  Its input is the cutout kernel's NHWC image: patch 1, kpad 8 (3 channels)."""
+
+    def __init__(self, name, state_dict, device):
+        res, layers, width, heads, embed = CLIP_RESNET_CONFIGS[name]
+        self.device = _resnet_device(device)
+        self.name = name
+        self.input_resolution, self.layers, self.width, self.heads, self.output_dim = res, layers, width, heads, embed
+        self.patch, self.kpad, self.grid = 1, 8, res
+        self.embed_width = 32 * width  # the attention pool's C
+        self.spatial = res // 32
+        self.tokens = self.spatial ** 2 + 1
+        sd, dev = state_dict, self.device
+        self.stem = [_Conv(sd, "visual.conv%d" % i, "visual.bn%d" % i, dev, dgrad=i > 1) for i in (1, 2, 3)]
+        self.w_stem1_f32 = _f32(self.stem[0].w_f32, dev)  # [width/2, 3, 3, 3]
+        self.blocks = []
+        for p, cin, planes, stride, ds in _resnet_blocks(name):
+            blk = {"cin": cin, "planes": planes, "stride": stride,
+                   "c1": _Conv(sd, p + "conv1", p + "bn1", dev), "c2": _Conv(sd, p + "conv2", p + "bn2", dev),
+                   "c3": _Conv(sd, p + "conv3", p + "bn3", dev), "ds": _Conv(sd, p + "downsample.0", p + "downsample.1", dev) if ds else None}
+            self.blocks.append(blk)
+        a = "visual.attnpool."
+        C = self.embed_width
+        self.pos = _f32(sd[a + "positional_embedding"], dev)
+        w_qkv = torch.cat([sd[a + "q_proj.weight"], sd[a + "k_proj.weight"], sd[a + "v_proj.weight"]])
+        self.w_qkv, self.w_qkv_t = _bf16(w_qkv, dev), _bf16(w_qkv.t(), dev)  # [3C, C], [C, 3C]
+        self.b_qkv = _f32(torch.cat([sd[a + "q_proj.bias"], sd[a + "k_proj.bias"], sd[a + "v_proj.bias"]]), dev)
+        self.w_c = _bf16(sd[a + "c_proj.weight"], dev)  # [E, C]
+        self.w_c_t = _f32(sd[a + "c_proj.weight"].t(), dev)  # [C, E] fp32 (cg_vit_proj_bwd's proj)
+        self.b_c = _f32(sd[a + "c_proj.bias"], dev)
+        assert C == heads * 64
+        self._init_graph_tower()
+
+    def _geometry(self):
+        """Per block: (spatial size of its input, of its output)."""
+        h = self.input_resolution // 4
+        out = []
+        for blk in self.blocks:
+            out.append((h, h // blk["stride"]))
+            h //= blk["stride"]
+        return out
+
+    def _new_workspace(self, n):
+        dev = self.device
+        b16 = lambda *s: torch.empty(*s, device=dev, dtype=torch.bfloat16)
+        f32 = lambda *s: torch.empty(*s, device=dev, dtype=torch.float32)
+        h1 = self.input_resolution // 2
+        M1 = n * h1 * h1
+        ws = {"stem": [b16(M1, c.w.shape[0]) for c in self.stem], "x0": b16(n * (h1 // 2) ** 2, self.stem[2].w.shape[0]), "blocks": []}
+        col = M1 * max([c.k for c in self.stem] + [c.kt for c in self.stem[1:]])  # im2col rows: the largest of every 3x3 convolution
+        grads = {}  # fp32 gradient and its bf16 copy per activation shape; a block without downsample updates its gradient in place
+        scratch = 0
+        for blk, (hi, ho) in zip(self.blocks, self._geometry()):
+            Mi, Mo = n * hi * hi, n * ho * ho
+            c1, c2, c3 = blk["c1"], blk["c2"], blk["c3"]
+            ws["blocks"].append({"a1": b16(Mi, c1.w.shape[0]), "a2": b16(Mi, c2.w.shape[0]), "y": b16(Mo, c3.w.shape[0])})
+            col = max(col, Mi * c2.k, Mi * c2.kt)
+            scratch = max(scratch, Mo * c2.w.shape[0], Mo * _r128(blk["cin"]), Mo * c3.w.shape[0], Mi * c2.w.shape[0])
+            for rows, cols in ((Mo, c3.w.shape[0]), (Mi, _r128(blk["cin"]))):
+                if (rows, cols) not in grads:
+                    grads[(rows, cols)] = (f32(rows, cols), b16(rows, cols))
+        ws["grads"] = grads
+        ws["col"] = b16(col)
+        # bf16 scratch of the block: pooled a2 / pooled x / the downsample's output (forward), d(pooled a2) (backward)
+        ws["s_pa2"], ws["s_px"], ws["s_idn"] = b16(scratch), b16(scratch), b16(scratch)
+        ws["s_dz"] = b16(scratch)
+        ws["s_dpx"] = f32(scratch)
+        C, T = self.embed_width, self.tokens
+        ws.update({"tok": b16(n * T, C), "qkv": b16(n * T, 3 * C), "ctx": b16(n * T, C), "lse": f32(n, self.heads, T),
+                   "dy": f32(n, C), "dctx": b16(n * T, C), "dqkv": b16(n * T, 3 * C), "delta": f32(n, self.heads, T), "dtok": f32(n * T, C)})
+        ws["dz_stem"] = [b16(M1, c.w.shape[0]) for c in self.stem]
+        return ws
+
+    @staticmethod
+    def _view(buf, rows, cols):
+        return buf[: rows * cols].view(rows, cols)
+
+    def _im2col(self, ws, x, n, h, C, stride, kpad):
+        P = _lib.ptr
+        ho = (h - 1) // stride + 1
+        col = self._view(ws["col"], n * ho * ho, kpad)
+        _lib.call("cg_im2col3x3_nhwc", P(x), n, h, h, C, x.stride(0), stride, kpad, P(col))
+        return col
+
+    def _forward_body(self, ws, n):
+        P, C_ = _lib.ptr, _lib.call
+        relu = gemm_bf16_tn_relu
+        R = self.input_resolution
+        h1 = R // 2
+        x = ws["patches"].view(n * R * R, self.kpad)
+        s1, s2, s3 = ws["stem"]
+        c1, c2, c3 = self.stem
+        relu(self._im2col(ws, x, n, R, 3, 2, c1.k), c1.w, _lib.EPI_BIAS_RELU_BF16, bias=c1.b, out=s1)
+        relu(self._im2col(ws, s1, n, h1, c2.cin, 1, c2.k), c2.w, _lib.EPI_BIAS_RELU_BF16, bias=c2.b, out=s2)
+        relu(self._im2col(ws, s2, n, h1, c3.cin, 1, c3.k), c3.w, _lib.EPI_BIAS_RELU_BF16, bias=c3.b, out=s3)
+        C_("cg_avgpool2x2_nhwc_fwd", P(s3), n, h1, h1, s3.shape[1], P(ws["x0"]))
+        x = ws["x0"]
+        for blk, L, (hi, ho) in zip(self.blocks, ws["blocks"], self._geometry()):
+            b1, b2, b3, ds = blk["c1"], blk["c2"], blk["c3"], blk["ds"]
+            relu(x[:, : b1.k], b1.w, _lib.EPI_BIAS_RELU_BF16, bias=b1.b, out=L["a1"])
+            relu(self._im2col(ws, L["a1"], n, hi, b2.cin, 1, b2.k), b2.w, _lib.EPI_BIAS_RELU_BF16, bias=b2.b, out=L["a2"])
+            pa2 = L["a2"]
+            if blk["stride"] > 1:
+                pa2 = self._view(ws["s_pa2"], n * ho * ho, L["a2"].shape[1])
+                C_("cg_avgpool2x2_nhwc_fwd", P(L["a2"]), n, hi, hi, pa2.shape[1], P(pa2))
+            idn = x
+            if ds is not None:
+                px = x
+                if blk["stride"] > 1:
+                    px = self._view(ws["s_px"], n * ho * ho, x.shape[1])
+                    C_("cg_avgpool2x2_nhwc_fwd", P(x), n, hi, hi, x.shape[1], P(px))
+                idn = self._view(ws["s_idn"], n * ho * ho, ds.w.shape[0])
+                gemm_bf16_tn(px[:, : ds.k], ds.w, _lib.EPI_BIAS_BF16, bias=ds.b, out=idn)
+            relu(pa2[:, : b3.k], b3.w, _lib.EPI_BIAS_RESID_RELU_BF16, bias=b3.b, resid=idn, out=L["y"])
+            x = L["y"]
+        # attention pool: tokens -> packed q|k|v -> attention -> c_proj of the query row 0 of every image
+        C, T = self.embed_width, self.tokens
+        C_("cg_resnet_attnpool_fwd", P(x), P(self.pos), n, T - 1, C, P(ws["tok"]))
+        gemm_bf16_tn(ws["tok"], self.w_qkv, _lib.EPI_BIAS_BF16, bias=self.b_qkv, out=ws["qkv"])
+        C_("cg_attention_fwd", P(ws["qkv"]), n, T, self.heads, P(ws["ctx"]), P(ws["lse"]))
+        ws["emb"].zero_()
+        gemm_bf16_tn(ws["ctx"].view(n, T * C)[:, :C], self.w_c, _lib.EPI_BIAS_RESID_F32, bias=self.b_c, out=ws["emb"], aux=ws["emb"])
+
+    def _backward_body(self, ws, n):
+        P, C_ = _lib.ptr, _lib.call
+        relu = gemm_bf16_tn_relu
+        C, T, E = self.embed_width, self.tokens, self.output_dim
+        C_("cg_vit_proj_bwd", P(ws["demb"]), P(self.w_c_t), n, C, E, P(ws["dy"]))
+        C_("cg_resnet_attnpool_dctx", P(ws["dy"]), n, T, C, P(ws["dctx"]))
+        C_("cg_attention_bwd", P(ws["qkv"]), P(ws["ctx"]), P(ws["dctx"]), P(ws["lse"]), n, T, self.heads, P(ws["dqkv"]), P(ws["delta"]))
+        gemm_bf16_tn(ws["dqkv"], self.w_qkv_t, _lib.EPI_F32, out=ws["dtok"])
+        y_last = ws["blocks"][-1]["y"]
+        g32, g16 = ws["grads"][tuple(y_last.shape)]
+        C_("cg_resnet_attnpool_bwd", P(ws["dtok"]), P(y_last), n, T - 1, C, P(g32), P(g16))
+        geo = self._geometry()
+        for i in reversed(range(len(self.blocks))):
+            blk, L, (hi, ho) = self.blocks[i], ws["blocks"][i], geo[i]
+            b1, b2, b3, ds = blk["c1"], blk["c2"], blk["c3"], blk["ds"]
+            x_in = ws["blocks"][i - 1]["y"] if i else ws["x0"]
+            g32_in, g16_in = ws["grads"][(x_in.shape[0], x_in.shape[1])]
+            # conv3 (1x1) dgrad; through the pool into a2's ReLU
+            if blk["stride"] > 1:
+                dp = self._view(ws["s_dz"], n * ho * ho, L["a2"].shape[1])
+                gemm_bf16_tn(g16[:, : b3.kt], b3.wt, _lib.EPI_BF16, out=dp)
+                dz2 = self._view(ws["s_pa2"], n * hi * hi, L["a2"].shape[1])
+                C_("cg_avgpool2x2_nhwc_bwd", P(dp), 0, P(L["a2"]), n, hi, hi, dz2.shape[1], P(dz2), 0)
+            else:
+                dz2 = self._view(ws["s_pa2"], n * hi * hi, L["a2"].shape[1])
+                relu(g16[:, : b3.kt], b3.wt, _lib.EPI_DRELU_BF16, mask=L["a2"], out=dz2)
+            # conv2 (3x3) dgrad as a convolution of dz2 with the flipped weights, into a1's ReLU
+            dz1 = self._view(ws["s_dz"], n * hi * hi, L["a1"].shape[1])
+            relu(self._im2col(ws, dz2, n, hi, b2.cout, 1, b2.kt), b2.wt, _lib.EPI_DRELU_BF16, mask=L["a1"], out=dz1)
+            # the identity path's gradient (in place when the block has no downsample), then conv1's dgrad joins it
+            if ds is not None:
+                if blk["stride"] > 1:
+                    dpx = self._view(ws["s_dpx"], n * ho * ho, g32_in.shape[1])
+                    gemm_bf16_tn(g16[:, : ds.kt], ds.wt, _lib.EPI_F32, out=dpx)
+                    C_("cg_avgpool2x2_nhwc_bwd", P(dpx), 1, None, n, hi, hi, dpx.shape[1], P(g32_in), 1)
+                else:
+                    gemm_bf16_tn(g16[:, : ds.kt], ds.wt, _lib.EPI_F32, out=g32_in)
+            relu(dz1[:, : b1.kt], b1.wt, _lib.EPI_RESID_DRELU, resid=g32_in, mask=x_in if i else None, out=g32_in, out_bf16=g16_in)
+            g32, g16 = g32_in, g16_in
+        # stem: the pool, then conv3 and conv2 (3x3, stride 1) as flipped convolutions, conv1 (stride 2) by its gather kernel
+        R = self.input_resolution
+        h1 = R // 2
+        s1, s2, s3 = ws["stem"]
+        c1, c2, c3 = self.stem
+        d1, d2, d3 = ws["dz_stem"]
+        C_("cg_avgpool2x2_nhwc_bwd", P(g32), 1, P(s3), n, h1, h1, s3.shape[1], P(d3), 0)
+        relu(self._im2col(ws, d3, n, h1, c3.cout, 1, c3.kt), c3.wt, _lib.EPI_DRELU_BF16, mask=s2, out=d2)
+        relu(self._im2col(ws, d2, n, h1, c2.cout, 1, c2.kt), c2.wt, _lib.EPI_DRELU_BF16, mask=s1, out=d1)
+        C_("cg_conv3x3s2_dgrad", P(d1), n, R, R, c1.cout, d1.stride(0), P(self.w_stem1_f32), 3, self.kpad, P(ws["dpatch"]))
+
+    def flops_fwd_bwd(self, n):
+        """Algorithmic FLOPs (2 x MAC) of forward + input gradient for n images, unpadded channel counts."""
+        R, h1 = self.input_resolution, self.input_resolution // 2
+        conv = lambda m, cin, cout, k: 2 * m * cin * cout * k * k  # noqa: E731
+        fwd = sum(conv(h1 * h1, c.cin, c.cout, 3) for c in self.stem)
+        bwd = sum(conv(h1 * h1, c.cin, c.cout, 3) for c in self.stem)  # conv1's dgrad: same MACs
+        for blk, (hi, ho) in zip(self.blocks, self._geometry()):
+            cin, p = blk["cin"], blk["planes"]
+            f = conv(hi * hi, cin, p, 1) + conv(hi * hi, p, p, 3) + conv(ho * ho, p, 4 * p, 1)
+            if blk["ds"] is not None:
+                f += conv(ho * ho, cin, 4 * p, 1)
+            fwd += f
+            bwd += f
+        C, T, E = self.embed_width, self.tokens, self.output_dim
+        fwd += 6 * T * C * C + 4 * T * T * C + 2 * C * E
+        bwd += 6 * T * C * C + 8 * T * T * C + 2 * C * E
         return n * (fwd + bwd)
 
 
@@ -467,11 +820,16 @@ class CLIPModelB200:
     """Value type of the dict returned by ``load_clip_models`` (models.py:74-84)."""
 
     def __init__(self, name, state_dict=None, device="cuda", seed=1):
-        if name not in CLIP_CONFIGS:
-            raise ValueError("unsupported CLIP model %r: this path implements the ViT towers %s" % (name, sorted(CLIP_CONFIGS)))
         self.name = name
-        sd = state_dict if state_dict is not None else random_clip_state_dict(name, seed)
-        self.visual = _Visual(VisionTransformerB200(name, sd, device))
+        if name in CLIP_RESNET_CONFIGS:
+            _resnet_device(device)  # before the random init: the tower has no CPU path
+            sd = state_dict if state_dict is not None else random_clip_resnet_state_dict(name, seed)
+            self.visual = _Visual(ModifiedResNetB200(name, sd, device))
+        elif name in CLIP_CONFIGS:
+            sd = state_dict if state_dict is not None else random_clip_state_dict(name, seed)
+            self.visual = _Visual(VisionTransformerB200(name, sd, device))
+        else:
+            raise ValueError("unsupported CLIP model %r: this path implements %s" % (name, sorted(CLIP_CONFIGS) + sorted(CLIP_RESNET_CONFIGS)))
         # the text tower is built on the first encode_text (image-only use keeps its memory and load time): until then the
         # checkpoint's non-visual tensors stay where the caller put them (load_clip_models: host memory); random init is seeded
         self._seed, self._text = seed, None
@@ -535,13 +893,14 @@ def load_clip_models(model_names, device=None, allow_random_init=False):
     wdir = os.environ.get("CLIPGUIDE_B200_WEIGHTS")
     models = {}
     for i, name in enumerate(model_names):
-        if name not in CLIP_CONFIGS:
-            raise ValueError("unsupported CLIP model %r: this path implements the ViT towers %s" % (name, sorted(CLIP_CONFIGS)))
+        if name not in CLIP_CONFIGS and name not in CLIP_RESNET_CONFIGS:
+            raise ValueError("unsupported CLIP model %r: this path implements %s" % (name, sorted(CLIP_CONFIGS) + sorted(CLIP_RESNET_CONFIGS)))
         sd = None
         path = os.path.join(wdir, name.replace("/", "_") + ".pt") if wdir else None
         if path and os.path.exists(path):
             sd = torch.load(path, map_location="cpu")
-            _require_keys(sd, random_clip_state_dict_keys(name), path, "visual-tower")
+            keys = clip_resnet_state_dict_shapes(name) if name in CLIP_RESNET_CONFIGS else random_clip_state_dict_keys(name)
+            _require_keys(sd, keys, path, "visual-tower")
         elif not allow_random_init:
             raise FileNotFoundError(
                 "no weights for %r: set CLIPGUIDE_B200_WEIGHTS to a directory holding %s.pt (OpenAI CLIP state dict), or pass "

@@ -52,3 +52,33 @@ def gemm_bf16_tn(a, b, epilogue, bias=None, out=None, aux=None, pos=None, g2=0, 
         _lib.ptr(aux), out.stride(0), _lib.ptr(pos), g2,
     )
     return (out, aux) if epilogue == _lib.EPI_BIAS_QGELU_BF16 else out
+
+
+_RELU_EPILOGUES = (_lib.EPI_BIAS_RELU_BF16, _lib.EPI_BIAS_RESID_RELU_BF16, _lib.EPI_DRELU_BF16, _lib.EPI_RESID_DRELU)
+
+
+def gemm_bf16_tn_relu(a, b, epilogue, bias=None, resid=None, mask=None, out=None, out_bf16=None):
+    """cg_gemm_bf16_tn_relu: acc[M,N] = a[M,K] @ b[N,K]^T with one of the ReLU-network epilogues (CG_EPI_BIAS_RELU_BF16 ..
+    CG_EPI_RESID_DRELU in the header).  ``out`` (fp32 for RESID_DRELU, bf16 otherwise), ``resid``, ``mask`` and ``out_bf16`` share one
+    row stride; resid may be ``out`` itself (RESID_DRELU)."""
+    _lib.require_cuda(a, b, bias, resid, mask, out, out_bf16)
+    if epilogue not in _RELU_EPILOGUES:
+        raise _lib.ClipGuideError("gemm_bf16_tn_relu: %d is not a ReLU epilogue" % epilogue)
+    assert a.dtype == torch.bfloat16 and b.dtype == torch.bfloat16 and a.stride(-1) == 1 and b.stride(-1) == 1
+    M, K, N = a.shape[0], a.shape[1], b.shape[0]
+    assert b.shape[1] == K
+    f32 = epilogue == _lib.EPI_RESID_DRELU
+    _check_matrix("out", out, torch.float32 if f32 else torch.bfloat16, M, N, a.device)
+    for name, t in (("resid", resid), ("mask", mask), ("out_bf16", out_bf16)):
+        if t is None:
+            continue
+        dtype = torch.float32 if (f32 and name == "resid") else torch.bfloat16
+        _check_matrix(name, t, dtype, M, N, a.device)
+        if t.stride(0) != out.stride(0):
+            raise _lib.ClipGuideError("gemm_bf16_tn_relu: %s row stride %d != out row stride %d" % (name, t.stride(0), out.stride(0)))
+    if epilogue in (_lib.EPI_BIAS_RELU_BF16, _lib.EPI_BIAS_RESID_RELU_BF16):
+        if bias is None or bias.dtype != torch.float32 or not bias.is_contiguous() or bias.shape != (N,) or bias.device != a.device:
+            raise _lib.ClipGuideError("gemm_bf16_tn_relu: epilogue %d needs a contiguous fp32 bias of length %d on %s" % (epilogue, N, a.device))
+    _lib.call("cg_gemm_bf16_tn_relu", _lib.ptr(a), _lib.ptr(b), M, N, K, a.stride(0), b.stride(0), epilogue, _lib.ptr(bias), _lib.ptr(resid),
+              _lib.ptr(mask), _lib.ptr(out), _lib.ptr(out_bf16), out.stride(0))
+    return out

@@ -180,6 +180,51 @@ int cg_gemm_bf16_tn(const void* A, const void* B, int M, int N, int K, int64_t l
 #define CG_GEMM_TILE_PAIR_256x256 2 /* two CTAs of a cluster share one 256 x 256 tile */
 int cg_gemm_tile_variant(int M, int N, int K, int epilogue);
 
+/* ------------------------------------------------------------------ CLIP ModifiedResNet ---- */
+/* The OpenAI CLIP ModifiedResNet image tower (clip/model.py ModifiedResNet: the RN101 of chosen_clip_models, config.py:41, reached
+ * through embed_image like the ViTs) on NHWC bf16 activations, rows [N*H*W, C].  BatchNorm (eval) is folded into the convolution
+ * weights and biases at load, so each convolution is a GEMM plus bias: a 1x1 convolution reads the activation rows as its A operand,
+ * a 3x3 convolution reads the rows cg_im2col3x3_nhwc builds.  The input gradient of a stride-1 3x3 convolution is the same convolution
+ * of the output gradient with the flipped, transposed weights W'[cin, (ky*3 + kx)*Cout + cout] = W[cout, cin, 2 - ky, 2 - kx]. */
+
+/* The GEMM epilogues of a ReLU network (cg_gemm_bf16_tn_relu; the mask tests follow torch's threshold_backward: 0 where the saved
+ * output is <= 0): */
+#define CG_EPI_BIAS_RELU_BF16 7        /* out_bf16 = relu(acc + bias)                           (stem convs, Bottleneck conv1/conv2) */
+#define CG_EPI_BIAS_RESID_RELU_BF16 8  /* out_bf16 = relu(acc + bias + resid_bf16)              (Bottleneck conv3 + identity)  */
+#define CG_EPI_DRELU_BF16 9            /* out_bf16 = acc * [mask_bf16 > 0]                      (dgrads into a ReLU output)     */
+#define CG_EPI_RESID_DRELU 10          /* out_f32 = (acc + resid_f32) * [mask_bf16 > 0] (no mask: 1; resid may alias out_f32),
+                                          out_bf16 = bf16(out_f32)                              (conv1 dgrad + identity gradient) */
+/* cg_gemm_bf16_tn with one of the epilogues 7-10: same operands, sizes and tile variants.  resid, mask and out_bf16 are addressed with
+ * ldo like out; bias (7, 8), resid (8, 10), mask (9; optional for 10) and out_bf16 (10) are given exactly when the epilogue reads or
+ * writes them, NULL otherwise.  out is fp32 for RESID_DRELU and bf16 otherwise. */
+int cg_gemm_bf16_tn_relu(const void* A, const void* B, int M, int N, int K, int64_t lda, int64_t ldb, int epilogue, const float* bias,
+                         const void* resid, const void* mask, void* out, void* out_bf16, int64_t ldo, void* stream);
+
+/* nn.Conv2d(C, *, 3, stride, padding=1)'s im2col rows: x [N,H,W] pixels of ldx bf16 values (the first C are the channels) ->
+ * out [N*Ho*Wo, kpad] bf16, column (ky*3 + kx)*C + c, zero for taps outside the image and for columns >= 9C.  Ho = (H-1)/stride + 1;
+ * stride 1 or 2; kpad a multiple of 64 and >= 9C; ldx % 8 == 0.  A pure copy. */
+int cg_im2col3x3_nhwc(const void* x, int N, int H, int W, int C, int64_t ldx, int stride, int kpad, void* out, void* stream);
+/* Input gradient of the stem's conv1 (3x3, stride 2, padding 1, no bias; the flip above needs stride 1): dy [N, Ho, Wo] pixels of lddy
+ * bf16 values (the first Cout are the channels), w [Cout, Cin, 3, 3] fp32 -> dx [N, H, W, kpad] fp32 (columns >= Cin zero): the
+ * CG_FMT_F32_PATCH layout with patch 1 that cg_cutouts_bwd and cg_patchify_bwd read.  Each pixel sums its (at most 4) output positions
+ * x Cout channels in a fixed order.  Cin <= 8, Cout <= 256. */
+int cg_conv3x3s2_dgrad(const void* dy, int N, int H, int W, int Cout, int64_t lddy, const float* w, int Cin, int kpad, float* dx, void* stream);
+/* nn.AvgPool2d(2) on NHWC bf16 rows (Bottleneck.avgpool, downsample[-1], the stem's pool): x [N,H,W,C] -> y [N,H/2,W/2,C], fp32 sums.
+ * H, W even, C % 8 == 0. */
+int cg_avgpool2x2_nhwc_fwd(const void* x, int N, int H, int W, int C, void* y, void* stream);
+/* Its gradient: dx [N,H,W,C] = 0.25 dy[n, y/2, x/2, c], times [mask > 0] when the bf16 mask [N,H,W,C] (a saved ReLU output) is given.
+ * dy fp32 (dy_f32) or bf16, dx fp32 (dx_f32) or bf16. */
+int cg_avgpool2x2_nhwc_bwd(const void* dy, int dy_f32, const void* mask, int N, int H, int W, int C, void* dx, int dx_f32, void* stream);
+/* AttentionPool2d's tokens: x [N*S, C] bf16 (the last stage's output, S = H*W), pos [S+1, C] fp32 ->
+ * tok [N*(S+1), C] bf16, tok[n,0] = mean_s x[n,s] + pos[0], tok[n,1+s] = x[n,s] + pos[1+s] (the A operand of the packed q|k|v
+ * projection; attention is cg_attention_fwd / _bwd with T = S+1).  C % 8 == 0. */
+int cg_resnet_attnpool_fwd(const void* x, const float* pos, int N, int S, int C, void* tok, void* stream);
+/* Its gradient through the last stage's ReLU: dtok [N*(S+1), C] fp32 -> g[n,s] = (dtok[n,1+s] + dtok[n,0]/S) * [x[n,s] > 0], fp32 g and
+ * its bf16 copy g_bf16, both [N*S, C]. */
+int cg_resnet_attnpool_bwd(const float* dtok, const void* x, int N, int S, int C, float* g, void* g_bf16, void* stream);
+/* The pool's output is attention row 0 only: dctx [N*T, C] bf16 = dy[n] (fp32 [N, C]) in row n*T, zero in every other row. */
+int cg_resnet_attnpool_dctx(const float* dy, int N, int T, int C, void* dctx, void* stream);
+
 /* Fused multi-head attention over packed qkv [Nimg*T, 3*D] bf16 (q | k | v, head h at column h*64), head_dim 64,
  * softmax scale 1/8.  ctx [Nimg*T, D] bf16, lse [Nimg, heads, T] fp32. */
 int cg_attention_fwd(const void* qkv, int Nimg, int T, int heads, void* ctx, float* lse, void* stream);
